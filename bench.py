@@ -67,6 +67,8 @@ WORKLOADS = {
 SPP_PER_FRAME = 64
 N_QUADS, TEX_SIZE = 224, 1024
 CPU_SAMPLE = dict(crop_frac=4, frames=1, paths=518400)  # centred crop of 1/4 x 1/4 of the image, ~0.5 M camera paths
+# --dump-outputs: at most this many pixels of the screenshot (2 Mi x (3 x f32 + f64 index) = 40 MiB), picked by a fixed seed
+DUMP_PIXELS, DUMP_SEED = 1 << 21, 0
 
 
 def build_scene(rt, name):
@@ -193,6 +195,18 @@ def microbench(extend_blocks_per_sm):
         out["issue_tops"][kname] = L.mb_issue_tops(kind, 4096)
     out["stream_copy_gbs"] = L.mb_stream_gbs(1 << 30)
     return out
+
+
+def dump_outputs(out_dir, shot):
+    """What the timed path hands its caller, the RGB8 screenshot (H, W, 3), as .npy files that two builds can be
+    compared on: screenshot.npy holds the RGB values (float32, one row per pixel) of up to DUMP_PIXELS pixels drawn
+    without replacement by a fixed seed, screenshot_pixel_index.npy their row-major pixel indices (float64, ascending).
+    An image of at most DUMP_PIXELS pixels is written whole."""
+    os.makedirs(out_dir, exist_ok=True)
+    rgb = shot.reshape(-1, 3)
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(rgb.shape[0], size=min(rgb.shape[0], DUMP_PIXELS), replace=False))
+    np.save(os.path.join(out_dir, "screenshot.npy"), rgb[idx].astype(np.float32))
+    np.save(os.path.join(out_dir, "screenshot_pixel_index.npy"), idx.astype(np.float64))
 
 
 def pinned_copy(torch, a: np.ndarray):
@@ -618,6 +632,8 @@ def run_gpu(args, rt):
     sampler = ClockSampler(local_rank) if (rank == 0 and not os.environ.get("RT_BENCH_NO_CLOCKS")) else None
     m = R.timed(be, u, frames, args.steps, args.warmup, sampler)
     c = m["counters"]
+    if args.dump_outputs and rank == 0:   # the last timed step's image, still on the device
+        dump_outputs(args.dump_outputs, be.screenshot_fetch())
     e2e, shot = R.e2e(be, scene, u, frames, max(1, min(args.steps, 2)))
     gate = parity_gate(rt, be, scene, name, shot, frames, world) if rank == 0 else None
 
@@ -671,7 +687,9 @@ def run_gpu(args, rt):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3,
+                    help="timed steps of the line's `value`; the e2e leg times min(steps, 2), the config2 / config4 side "
+                         "blocks a fixed 3 / 2")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
@@ -682,7 +700,14 @@ def main():
                     help="default and contract: 4k (BASELINE config 5 at a quarter of its samples)")
     ap.add_argument("--split", default="frames", choices=["frames", "tiles"],
                     help="N > 1: frame-slice split + ncclReduce (default) or image-tile split + gather")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the screenshot of the last timed step to DIR/*.npy (see dump_outputs); GPU path only, "
+                         "the reference arm renders a crop at reduced spp that no build is compared on")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed (--impl ours)")
     rt = importlib.import_module("raytracing2-fork_b200")
     if args.impl == "reference":
         run_reference(args, rt)

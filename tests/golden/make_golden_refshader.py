@@ -1,6 +1,6 @@
 """Mint tests/golden/refshader_images.npz (+ refshader.json) from the REFERENCE'S OWN compute shader source.
 
-Needs /root/reference (run in the authoring container after `make -C oracle`): every image here is what
+Needs a reference checkout (RT_REFERENCE=<path> make -C oracle first): every image here is what
 RayTracing/Assets/Shaders/compute.glsl itself computes — rewritten syntactically by oracle/glsl2cpp.py,
 compiled against the reference's vendored glm, walking the node array the reference's BVH.h built
 (oracle/_ref/ref_host) — for the cases of tests/scenes.py::refshader_cases().  The GL driver's elementary
@@ -26,7 +26,7 @@ import scenes  # noqa: E402
 
 
 def main():
-    assert refshader.available(True), "oracle/_ref/libref_shader.so missing: make -C oracle (needs /root/reference)"
+    assert refshader.available(True), "oracle/_ref/libref_shader.so missing: make -C oracle (needs RT_REFERENCE)"
     assert oracle.have_ref_host(), "oracle/_ref/ref_host missing"
     meta, images = {}, {}
     for name, (scene, u) in scenes.refshader_cases().items():

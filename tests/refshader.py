@@ -1,6 +1,6 @@
 """ctypes view of oracle/_ref/libref_shader*.so: the reference's OWN compute shader source, rewritten
 syntactically by oracle/glsl2cpp.py and compiled against the reference's own glm (oracle/ref_shader.cpp).
-TEST INFRASTRUCTURE ONLY; present only where /root/reference was available to `make -C oracle`."""
+TEST INFRASTRUCTURE ONLY; present only where a reference checkout (RT_REFERENCE) was available to `make -C oracle`."""
 import ctypes as C
 import importlib
 import os

@@ -103,6 +103,27 @@ def test_reference_arm_prints_the_contract_line():
     assert d["config"]["name"] == "config1" and "workload" in d["config"]
 
 
+def test_dump_outputs_is_a_fixed_sample_within_64_mb(tmp_path):
+    """--dump-outputs: a small image is written whole; a 4K one as the same seeded pixel sample every time, under
+    64 MB in all, each stored value the image's own."""
+    import numpy as np
+    small = np.arange(6 * 5 * 3, dtype=np.uint8).reshape(6, 5, 3)
+    bench.dump_outputs(str(tmp_path / "s"), small)
+    assert np.array_equal(np.load(tmp_path / "s" / "screenshot.npy"), small.reshape(-1, 3).astype(np.float32))
+    assert np.array_equal(np.load(tmp_path / "s" / "screenshot_pixel_index.npy"), np.arange(30, dtype=np.float64))
+    shot = np.random.default_rng(1).integers(0, 256, (2160, 3840, 3), dtype=np.uint8)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), shot)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["screenshot.npy", "screenshot_pixel_index.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 << 20
+    for f in files:
+        assert (tmp_path / "a" / f).read_bytes() == (tmp_path / "b" / f).read_bytes()
+    rgb, idx = np.load(tmp_path / "a" / "screenshot.npy"), np.load(tmp_path / "a" / "screenshot_pixel_index.npy")
+    assert rgb.dtype == np.float32 and idx.dtype == np.float64 and rgb.shape == (bench.DUMP_PIXELS, 3)
+    assert np.all(np.diff(idx) > 0) and np.array_equal(rgb, shot.reshape(-1, 3)[idx.astype(np.int64)])
+
+
 def test_microbench_library_is_built_by_build():
     """bench.py's `ceilings` block (the L2 / HBM gather and FP32-issue rates the roofline is measured against) needs
     tools/libmicrobench.so; __graft_entry__.build() must compile it, and it must export what bench.microbench binds."""

@@ -12,9 +12,9 @@ import pytest
 import oracle
 
 rt = importlib.import_module("raytracing2-fork_b200")
-DATA = "/root/reference/RayTracing/Data"
-needs_ref = pytest.mark.skipif(not (oracle.have_ref_host() and os.path.isdir(DATA)),
-                               reason="needs /root/reference and oracle/_ref/ref_host")
+DATA = os.path.join(os.environ.get("RT_REFERENCE", ""), "RayTracing", "Data")   # RT_REFERENCE: a reference checkout
+needs_ref = pytest.mark.skipif(not (oracle.have_ref_host() and os.environ.get("RT_REFERENCE") and os.path.isdir(DATA)),
+                               reason="needs a reference checkout (RT_REFERENCE) and oracle/_ref/ref_host")
 
 
 @needs_ref

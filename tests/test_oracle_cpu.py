@@ -1,5 +1,5 @@
 """CPU tests (no GPU): the oracle against the REAL reference host code (oracle/_ref/ref_host, compiled
-from /root/reference when present), against published known answers, against libm, and against the
+from a reference checkout when RT_REFERENCE names one), against published known answers, against libm, and against the
 committed golden fixtures in tests/golden/."""
 import ctypes as C
 import importlib
@@ -15,7 +15,7 @@ import oracle
 
 rt = importlib.import_module("raytracing2-fork_b200")
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-needs_ref = pytest.mark.skipif(not oracle.have_ref_host(), reason="oracle/_ref/ref_host not built (no /root/reference)")
+needs_ref = pytest.mark.skipif(not oracle.have_ref_host(), reason="oracle/_ref/ref_host not built (needs a reference checkout: RT_REFERENCE)")
 
 DEFINED_MATERIAL_FIELDS = {  # fields the reference's Material::make* actually writes (mesh.h:47-102)
     rt.MAT_DIFFUSE: ["color", "materialType", "textureIndex", "isEdgeHighlight"],
@@ -110,6 +110,31 @@ def test_rng_stream_matches_reference_host_copy(tmp_path):
         assert st.value == states[i]
         mism += np.float32(v) != floats[i]
     assert mism < 400
+
+
+def test_bvh_and_fixed_materials_match_stored_reference_output(tmp_path):
+    """Without a reference checkout: tests/golden/sleeping.rtsc.gz is what the reference itself wrote for
+    Data/sleeping (tests/golden/make_golden_assets.sh): its loader's triangles, the five fixed materials its main()
+    appends (rayTracing.cpp:1268-1283), and the node array and triangle order of its own BVH.h over those triangles.
+    The oracle's BVH restatement and the host library's fixed materials must reproduce them bit for bit."""
+    import gzip
+    path = tmp_path / "sleeping.rtsc"
+    path.write_bytes(gzip.open(os.path.join(GOLDEN, "sleeping.rtsc.gz"), "rb").read())
+    ref = oracle.read_rtsc(str(path))
+    assert ref["tris"].size == 372 and ref["nodes"].size == 713
+    o = oracle.OracleScene(ref["tris"], ref["mats"], ref["tex"])
+    assert o.nodes().tobytes() == ref["nodes"].tobytes()
+    perm, orig = o.permuted()
+    assert tri_equal(perm, ref["perm"])
+    assert tri_equal(ref["tris"][orig], perm)
+    s = rt.Scene()
+    red = s.add_fixed_materials()
+    ours, theirs = s.materials[red:], ref["mats"][-5:]
+    assert ours.size == 5
+    for i in range(5):
+        assert int(ours["materialType"][i]) == int(theirs["materialType"][i])
+        for f in DEFINED_MATERIAL_FIELDS[int(ours["materialType"][i])]:
+            assert ours[f][i].tobytes() == theirs[f][i].tobytes(), (i, f)
 
 
 # ------------------------------------------------------------------------------------------------ known answers

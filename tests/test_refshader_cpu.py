@@ -3,7 +3,7 @@
 oracle/_ref/libref_shader.so is RayTracing/Assets/Shaders/compute.glsl itself — rewritten syntactically by
 oracle/glsl2cpp.py, compiled with g++ -ffp-contract=off against the reference's vendored glm 0.9.9.7, run over
 the node array the reference's own BVH.h builds (oracle/_ref/ref_host).  It exists wherever `make -C oracle`
-saw /root/reference (this container; the built library travels to the GPU box).  The committed
+saw a reference checkout (RT_REFERENCE).  The committed
 tests/golden/refshader_images.npz are its outputs; the tests below hold
 
   * golden == reference shader, regenerated here           (skipped without the library)
@@ -51,7 +51,7 @@ def test_oracle_equals_reference_shader_golden(golden, name):
     assert not diff.any(), f"{name}: {int(diff.sum())} of {diff.size} floats differ from the reference shader"
 
 
-@pytest.mark.skipif(not refshader.available(True), reason="oracle/_ref/libref_shader.so not built (needs /root/reference)")
+@pytest.mark.skipif(not refshader.available(True), reason="oracle/_ref/libref_shader.so not built (needs a reference checkout: RT_REFERENCE)")
 @pytest.mark.parametrize("name", sorted(CASES))
 def test_golden_is_what_the_reference_shader_computes(golden, name):
     scene, u = CASES[name]
@@ -120,10 +120,11 @@ def test_oracle_equals_reference_shader_at_full_size(name):
     assert (zlib.crc32(img.tobytes()) & 0xffffffff) == big["crc"]
 
 
-_DATA = "/root/reference/RayTracing/Data"
+_DATA = os.path.join(os.environ.get("RT_REFERENCE", ""), "RayTracing", "Data")
 
 
-@pytest.mark.skipif(not (refshader.available(True) and os.path.isdir(_DATA)), reason="needs /root/reference and its harness")
+@pytest.mark.skipif(not (refshader.available(True) and os.environ.get("RT_REFERENCE") and os.path.isdir(_DATA)),
+                    reason="needs a reference checkout (RT_REFERENCE) and its harness")
 @pytest.mark.parametrize("model,container", [("robot", "cornell"), ("autumn_kitten", "none"), ("campfire", "cornell"),
                                              ("rin", "none"), ("sleeping", "cornell"), ("mccree", "none"),
                                              ("building", "none"), ("plants", "cornell"), ("toonHouse", "none")])
@@ -145,7 +146,7 @@ def test_real_assets_oracle_equals_reference_shader(model, container):
     assert np.unique(ref).size > 10
 
 
-@pytest.mark.skipif(not refshader.available(True), reason="oracle/_ref/libref_shader.so not built (needs /root/reference)")
+@pytest.mark.skipif(not refshader.available(True), reason="oracle/_ref/libref_shader.so not built (needs a reference checkout: RT_REFERENCE)")
 @pytest.mark.parametrize("seed", range(64))
 def test_fuzz_oracle_equals_reference_shader(seed):
     """Seeded random triangle soups (every material type, 1/3/4-channel non-power-of-two textures, out-of-range
@@ -159,7 +160,7 @@ def test_fuzz_oracle_equals_reference_shader(seed):
     assert np.unique(ref[..., :3]).size > 2   # not a blank image
 
 
-@pytest.mark.skipif(not refshader.available(True), reason="oracle/_ref/libref_shader.so not built (needs /root/reference)")
+@pytest.mark.skipif(not refshader.available(True), reason="oracle/_ref/libref_shader.so not built (needs a reference checkout: RT_REFERENCE)")
 def test_screenshot_from_reference_shader_frames():
     """screenshot() of rayTracing.cpp:184-259 rebuilt around the reference shader: frame f is one dispatch with
     frameIndex = f, read back as RGB8 (round to nearest), accumulated as float, divided by the frame count, clamped,
