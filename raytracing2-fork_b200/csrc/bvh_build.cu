@@ -381,7 +381,7 @@ __global__ void __launch_bounds__(256) k_refit(const rt_triangle* __restrict__ t
 }
 
 // --------------------------------------------------------------------------------------------- PLOC
-// search window of the clustering (RT_PLOC_RADIUS overrides, 1..64).  Measured on config 2 (profiles/r2_knobs_ab.txt):
+// search window of the clustering.  Measured on config 2 (profiles/r2_knobs_ab.txt):
 // radius 6 -> 7.13 wide-node visits per segment, 10 -> 7.24, 16 / 25 / 40 -> slightly MORE visits and a slower build.
 constexpr int kPlocRadiusDefault = 6;
 
@@ -1055,8 +1055,8 @@ cudaError_t build_lbvh(const BuildArgs& a, cudaStream_t st, uint64_t* launches) 
         int32_t* parentOf = reinterpret_cast<int32_t*>(a.centroid);     // centroids are dead after k_morton: 16n bytes
         uint32_t* innerCount = reinterpret_cast<uint32_t*>(a.centroid) + n;
         int32_t* leafParent = reinterpret_cast<int32_t*>(a.flags);      // n + 1 words, free since the scan moved into the merge kernel
-        const LeafPolicy pol{a.leaf_cb > 0.0f ? a.leaf_cb : 0.35f, a.leaf_max_tris >= 1 ? (a.leaf_max_tris < 8 ? a.leaf_max_tris : 8) : 4};
-        const int radius = a.ploc_radius > 0 ? (a.ploc_radius < 64 ? a.ploc_radius : 64) : kPlocRadiusDefault;
+        const LeafPolicy pol{0.35f, 4};
+        const int radius = kPlocRadiusDefault;
         uint32_t* ctl = a.hist;                           // the histograms are dead after the sort
         unsigned long long* tileState = reinterpret_cast<unsigned long long*>(a.hist + kCtlWords);
         k_ploc_init<<<nb(n, 256), 256, 0, st>>>(a.tris, a.vals[0], n, a.bounds, a.boxes, cluster[0], height); L++; RT_DBG();
@@ -1090,14 +1090,13 @@ cudaError_t build_lbvh(const BuildArgs& a, cudaStream_t st, uint64_t* launches) 
             }
         }
         k_ploc_depth<<<1, 32, 0, st>>>(height, maxDepth); L++; RT_DBG();
-        // depth-first positions: of the inner nodes (their index in memory when dfs_layout is on), of the triangles in
+        // depth-first positions: of the inner nodes (their index in memory), of the triangles in
         // front of every subtree, and of every triangle (the order of the triangle records: leaves are contiguous runs)
-        int32_t* dfs = reinterpret_cast<int32_t*>(a.centroid) + 2 * (size_t)n;
+        order = reinterpret_cast<int32_t*>(a.centroid) + 2 * (size_t)n;
         firstTri = reinterpret_cast<int32_t*>(a.centroid) + 3 * (size_t)n;
         triPos = reinterpret_cast<int32_t*>(a.vals[1]);  // the cluster list that lived here is dead
-        k_dfs_order<<<nb(n - 1, 256), 256, 0, st>>>(n, a.children, parentOf, innerCount, dfs, firstTri); L++; RT_DBG();
+        k_dfs_order<<<nb(n - 1, 256), 256, 0, st>>>(n, a.children, parentOf, innerCount, order, firstTri); L++; RT_DBG();
         k_tri_order<<<nb(n, 256), 256, 0, st>>>(n, a.children, parentOf, leafParent, innerCount, triPos); L++; RT_DBG();
-        if (a.dfs_layout) order = dfs;
     } else {
         if (n >= 2) {
             k_hierarchy<<<nb(n - 1, 256), 256, 0, st>>>(a.keys[0], n, a.children, a.parent); L++; RT_DBG();

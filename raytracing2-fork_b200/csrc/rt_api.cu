@@ -109,20 +109,9 @@ struct rt_ctx {
     rt_config cfg{};
     int sm_count = 148;
     int extend_blocks_per_sm = 4;
-    int leaf_vote = 14, refill = 8, node_steps = 4;
-    int node_steps_wide = 2, extend_blocks_per_sm_wide = 8;
-    int use_ploc = 1, dfs_layout = 1, speculative = 1, shade_blocks_per_sm = 64;
-    int shade_defer_bounces = 1;   // RT_SHADE_DEFER_BOUNCES: with RT_SHADE_DEFER=3, a textured scene defers bounces below this
-    int shade_defer_batch = 3;     // RT_SHADE_DEFER_BATCH: windows per deferred reservation at bounce 0 (1 .. 3)
-    int shade_defer_batch_later = 3;  // RT_SHADE_DEFER_BATCH_LATER: ... at the later bounces
-    int shade_defer = 3;           // RT_SHADE_DEFER: k_shade appends its survivors one window late (0 never, 1 bounce 0, 2 always, 3 auto)
-    int top_smem = 0;              // RT_EXT_TOP=1: k_extend keeps the top four levels of the wide tree in shared memory
-    int leaf_max_tris = 0;         // RT_LEAF_MAX: most triangles per leaf (0 = builder default)
-    float leaf_cb = 0.0f;          // RT_LEAF_CB: SAH cost of a box test relative to a triangle test (0 = builder default)
-    int ploc_radius = 0;           // RT_PLOC_RADIUS: search window of the clustering (0 = the builder's default)
-    int force_widen = 0;           // RT_EXT_WIDEN=1: every launch uses the widened slab test (debugging aid)
+    int extend_blocks_per_sm_wide = 8;
+    int use_ploc = 1, shade_blocks_per_sm = 64;
     int hooks_thread = 0;          // RT_HOOKS=thread: parity hooks walk the binary tree per thread (preview's code path)
-    int extend_blocks_per_sm_top = 8;
     int bvh_width = 4;             // 4: k_extend walks 4-wide nodes collapsed from the binary tree; 2: the binary tree (RT_BVH_WIDTH)
     DevBuf d_wide_count;           // [0] wide nodes written, [1] worst-case traversal stack entries (k_collapse4)
     uint32_t wide_nodes = 0;
@@ -160,7 +149,6 @@ struct rt_ctx {
     float4* p_shade = nullptr;
     int32_t* p_orig = nullptr;
     size_t bvh_hot_bytes = 0;  // (wide or binary) nodes + tri_geom + tri_orig
-    int l2_persist = 1;
     float grid[6] = {0, 0, 0, 1, 1, 1};
     // wavefront
     DevBuf d_path[6], d_hit, d_contrib, d_accum, d_pixrng, d_counts, d_stats, d_image, d_sum, d_out, d_rows;
@@ -230,26 +218,15 @@ bool widen_needed(const rt_ctx* ctx, const rt_uniforms& u) {
 Launcher make_launcher(rt_ctx* ctx, const rt_uniforms* u = nullptr) {
     Launcher L;
     L.st = ctx->stream;
-    L.top_smem = ctx->top_smem != 0;
-    L.widen_primary = (u && !ctx->force_widen) ? widen_needed(ctx, *u) : true;
-    L.widen_always = ctx->force_widen != 0;
+    L.widen_primary = u ? widen_needed(ctx, *u) : true;
     L.hooks_thread = ctx->hooks_thread != 0;
 
     L.sm_count = ctx->sm_count;
     L.rng_mode = ctx->cfg.rng_mode;
     L.instrument = ctx->cfg.instrument != 0;
     L.extend_grid = ctx->sm_count * ctx->extend_blocks_per_sm;
-    L.extend_grid_wide = ctx->sm_count * (ctx->top_smem ? ctx->extend_blocks_per_sm_top : ctx->extend_blocks_per_sm_wide);
-    L.node_steps_wide = ctx->node_steps_wide;
-    L.leaf_vote = ctx->leaf_vote;
-    L.refill = ctx->refill;
-    L.node_steps = ctx->node_steps;
-    L.speculative = ctx->speculative != 0;
+    L.extend_grid_wide = ctx->sm_count * ctx->extend_blocks_per_sm_wide;
     L.shade_blocks_per_sm = ctx->shade_blocks_per_sm;
-    L.shade_defer = ctx->shade_defer;
-    L.shade_defer_batch = ctx->shade_defer_batch;
-    L.shade_defer_bounces = ctx->shade_defer_bounces;
-    L.shade_defer_batch_later = ctx->shade_defer_batch_later;
     L.kernel_launches = &ctx->kernel_launches;
     L.extend_launches = &ctx->extend_launches;
     L.ev_pool = ctx->events.data();
@@ -292,7 +269,7 @@ SceneView make_view(rt_ctx* ctx) {
 // a LOSS when the arena does not fit (config 4, 960 MB: a 10 % hitRatio window with streaming misses made
 // the step 18 % slower), so the window is set only when the whole arena fits the persisting carve-out.
 void apply_l2_window(rt_ctx* ctx) {
-    if (!ctx->l2_persist || !ctx->hot_base || ctx->bvh_hot_bytes == 0) return;
+    if (!ctx->hot_base || ctx->bvh_hot_bytes == 0) return;
     if (ctx->l2_max_persist < 0) {  // device limits, queried once (cudaGetDeviceProperties costs milliseconds)
         int v = 0;
         ctx->l2_max_persist = cudaDeviceGetAttribute(&v, cudaDevAttrMaxPersistingL2CacheSize, ctx->cfg.device) == cudaSuccess ? v : 0;
@@ -597,9 +574,8 @@ int rt_create(rt_ctx** out, const rt_config* cfg) {
         return fail(nullptr, RT_ERR_CUDA, m);
     }
     ctx->stream = ctx->own_stream;
-    ctx->extend_blocks_per_sm = wf_extend_blocks_per_sm(cfg->instrument != 0, false, false);
-    ctx->extend_blocks_per_sm_wide = wf_extend_blocks_per_sm(cfg->instrument != 0, true, false);
-    ctx->extend_blocks_per_sm_top = wf_extend_blocks_per_sm(false, true, true);
+    ctx->extend_blocks_per_sm = wf_extend_blocks_per_sm(cfg->instrument != 0, false);
+    ctx->extend_blocks_per_sm_wide = wf_extend_blocks_per_sm(cfg->instrument != 0, true);
     {
         // Path slots: fewer, larger wavefronts amortise the drain of the persistent kernels (config 2: 8 lanes
         // per pixel 1203 ms/step, 64 lanes 1057 ms; round 2: 128 Mi slots 744.8 ms, 512 Mi — the whole 4-frame
@@ -610,30 +586,12 @@ int rt_create(rt_ctx** out, const rt_config* cfg) {
             ctx->default_budget = std::min<uint64_t>(ctx->default_budget, (uint64_t)(freeB * 0.4) / 128u);
         if (ctx->default_budget < (1u << 20)) ctx->default_budget = 1u << 20;
     }
-    // tuning knobs of the persistent traversal kernel (defaults chosen from ncu runs, DESIGN.md §6)
-    if (const char* e1 = getenv("RT_EXT_LEAF_VOTE")) ctx->leaf_vote = std::max(1, std::min(32, atoi(e1)));
-    if (const char* e2 = getenv("RT_EXT_REFILL")) ctx->refill = std::max(1, std::min(32, atoi(e2)));
-    if (const char* e10 = getenv("RT_L2_PERSIST")) ctx->l2_persist = atoi(e10);
-    if (const char* e19 = getenv("RT_SHADE_DEFER_BOUNCES")) ctx->shade_defer_bounces = std::max(0, std::min(64, atoi(e19)));
-    if (const char* e17 = getenv("RT_SHADE_DEFER_BATCH")) ctx->shade_defer_batch = std::max(1, std::min(3, atoi(e17)));
-    if (const char* e18 = getenv("RT_SHADE_DEFER_BATCH_LATER")) ctx->shade_defer_batch_later = std::max(1, std::min(3, atoi(e18)));
-    if (const char* e16 = getenv("RT_SHADE_DEFER")) ctx->shade_defer = std::max(0, std::min(3, atoi(e16)));
+    // switches that keep the fallback and test-only paths reachable (README)
     if (const char* e9 = getenv("RT_SHADE_BLOCKS_PER_SM")) ctx->shade_blocks_per_sm = std::max(1, std::min(256, atoi(e9)));
     if (const char* e8 = getenv("RT_MAX_PATHS_MI")) ctx->default_budget = (uint64_t)std::max(1, atoi(e8)) << 20;
-    if (const char* e7 = getenv("RT_EXT_SPEC")) ctx->speculative = atoi(e7);
-    if (const char* e6 = getenv("RT_BVH_LAYOUT")) ctx->dfs_layout = strcmp(e6, "creation") != 0;
     if (const char* e9 = getenv("RT_BVH_WIDTH")) ctx->bvh_width = atoi(e9) == 4 ? 4 : 2;
     if (const char* e5 = getenv("RT_BVH_BUILDER")) ctx->use_ploc = strcmp(e5, "lbvh") != 0;
-    if (const char* e4 = getenv("RT_EXT_NODE_STEPS")) ctx->node_steps = std::max(1, std::min(16, atoi(e4)));
-    if (const char* e3 = getenv("RT_EXT_BLOCKS_PER_SM"))
-        ctx->extend_blocks_per_sm = ctx->extend_blocks_per_sm_wide = ctx->extend_blocks_per_sm_top = std::max(1, std::min(32, atoi(e3)));
-    if (const char* e11 = getenv("RT_EXT_TOP")) ctx->top_smem = atoi(e11);
-    if (const char* e15 = getenv("RT_EXT_WIDEN")) ctx->force_widen = atoi(e15);
-    if (const char* e17 = getenv("RT_LEAF_MAX")) ctx->leaf_max_tris = std::max(0, std::min(8, atoi(e17)));
-    if (const char* e18 = getenv("RT_LEAF_CB")) ctx->leaf_cb = (float)atof(e18);
-    if (const char* e16 = getenv("RT_PLOC_RADIUS")) ctx->ploc_radius = std::max(0, std::min(64, atoi(e16)));
     if (const char* e14 = getenv("RT_HOOKS")) ctx->hooks_thread = strcmp(e14, "thread") == 0;
-    if (const char* e10 = getenv("RT_EXT_NODE_STEPS_WIDE")) ctx->node_steps_wide = std::max(1, std::min(4, atoi(e10)));
     if (ctx->d_stats.reserve(4 * sizeof(unsigned long long)) != cudaSuccess ||
         cudaMemsetAsync(ctx->d_stats.p, 0, 4 * sizeof(unsigned long long), ctx->stream) != cudaSuccess) {
         delete ctx;
@@ -786,10 +744,6 @@ int rt_scene_build(rt_ctx* ctx) {
     a.tris = ctx->d_tris.as<rt_triangle>();
     a.n = n;
     a.use_ploc = ctx->use_ploc;
-    a.dfs_layout = ctx->dfs_layout;
-    a.ploc_radius = ctx->ploc_radius;
-    a.leaf_max_tris = ctx->leaf_max_tris;
-    a.leaf_cb = ctx->leaf_cb;
     a.centroid = ctx->d_centroid.as<float4>();
     a.bounds = ctx->d_bounds.as<uint32_t>();
     for (int i = 0; i < 2; i++) {
@@ -1082,7 +1036,7 @@ int rt_get_counters(rt_ctx* ctx, rt_counters* out) {
         out->bvh_bytes = (uint64_t)ctx->wide_nodes * 64 + (uint64_t)ctx->n_tris * 48;
         out->bvh_depth = (uint64_t)ctx->wide_depth;
         out->bvh_width = 4;
-        out->extend_blocks_per_sm = (uint64_t)(ctx->top_smem ? ctx->extend_blocks_per_sm_top : ctx->extend_blocks_per_sm_wide);
+        out->extend_blocks_per_sm = (uint64_t)ctx->extend_blocks_per_sm_wide;
         out->bvh_stack_need = ctx->wide_stack_need;
     }
     return RT_OK;

@@ -13,10 +13,6 @@ struct BuildArgs {
     const rt_triangle* tris;  // device copy of the caller's array (original order)
     int n;
     int use_ploc;             // 1 = PLOC hierarchy (default), 0 = Karras LBVH
-    int dfs_layout;           // 1 = store PLOC nodes in depth-first order
-    int ploc_radius;          // search window of the clustering, 0 = default
-    int leaf_max_tris;        // most triangles a leaf may hold (PLOC; 0 = default 4, 1 = one triangle per leaf)
-    float leaf_cb;            // SAH cost of a box test relative to a triangle test (0 = default)
     float4* centroid;         // n
     uint32_t* bounds;         // 12 order-preserving uints
     uint64_t* keys[2];        // n each
@@ -127,20 +123,9 @@ struct Launcher {
     bool instrument;
     int extend_grid;   // persistent k_extend grid: SMs x resident blocks per SM
     int extend_grid_wide;  // the same for the 4-wide variant (more registers)
-    int node_steps_wide;   // node steps per vote of the 4-wide variant
-    int leaf_vote;     // k_extend: leaf step when this many lanes wait at a leaf
-    int refill;        // k_extend: refill when this many lanes are idle
-    int node_steps;    // k_extend: node steps per vote
-    bool speculative;  // k_extend: postponed-leaf variant
-    bool top_smem;     // k_extend (4-wide): root + three levels of the tree staged in shared memory
-    bool widen_always;   // debugging aid: widened slab test on every bounce
     bool widen_primary;  // camera rays may start far outside the quantisation grid (rt_scene.cuh, slab1)
     bool hooks_thread; // parity hooks walk the binary tree per thread instead of running k_extend
     int shade_blocks_per_sm;  // grid-stride k_shade: blocks per SM
-    int shade_defer_bounces;      // auto policy: textured scenes defer the first this-many bounces
-    int shade_defer_batch;        // windows per deferred reservation at bounce 0 (1 .. 3)
-    int shade_defer_batch_later;  // ... at the later bounces
-    int shade_defer;          // k_shade's deferred queue append: 0 never, 1 at bounce 0, 2 at every bounce, 3 auto
     uint64_t* kernel_launches;
     uint64_t* extend_launches;
     // optional per-class device timing
@@ -151,7 +136,7 @@ struct Launcher {
     bool timing;
 };
 
-int wf_extend_blocks_per_sm(bool instrument, bool wide, bool top);
+int wf_extend_blocks_per_sm(bool instrument, bool wide);
 cudaError_t wf_clear_accum(const Launcher& L, const WaveBuffers& wb, long long entries);
 cudaError_t wf_seed_pixels(const Launcher& L, const SceneView& sc, const WaveBuffers& wb, const FrameParams& fp);
 cudaError_t wf_render_batch(const Launcher& L, const SceneView& sc, const WaveBuffers& wb, const FrameParams& fp);

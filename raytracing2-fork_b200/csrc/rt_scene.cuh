@@ -58,46 +58,20 @@ constexpr float kGuardCells = 0.125f;
 
 // 256-bit read-only global load (sm_100a: LDG.E.ENL2.256.CONSTANT): one instruction, one L1TEX
 // wavefront per lane for 32 bytes, where four 128-bit loads of a 64-byte record would cost four.
-// L1 eviction-priority hints of the two gathers of k_extend (PTX `.L1::evict_last` / `.L1::evict_first` /
-// `.L1::no_allocate`), empty by default; measured in profiles/r2_final_ab.txt.
-#ifndef RT_NODE_HINT
-#define RT_NODE_HINT ""
-#endif
-#ifndef RT_TRI_HINT
-#define RT_TRI_HINT ""
-#endif
+// (L1 eviction-priority hints on this load and on load_tri's measured neutral or slower: profiles/r2_final_ab.txt.)
 __device__ __forceinline__ void ldg256u(const void* p, uint32_t (&v)[8]) {
-    asm volatile("ld.global.nc" RT_NODE_HINT ".v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+    asm volatile("ld.global.nc.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                  : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
                  : "l"(p));
 }
-// exact uint16 -> float, two ways with identical results:
-//   I2F.U16   one instruction that reads the half register directly, but on the XU pipe: 16 lanes / clk / SM
-//             (tools/microbench.cu: 4.5 T/s against 17.8 T/s FFMA instructions);
-//   magic     splice the 16 bits into the mantissa of 2^23 (one PRMT / LOP3 on the ALU pipe, 64 lanes / clk) and
-//             subtract 2^23 (one FADD on the FMA pipe, 128 lanes / clk, 75 % idle in k_extend).
-// A 4-wide visit converts 24 planes; all on XU that is 192 pipe cycles per warp against ~131 issue slots — ncu round 2:
-// XU 54 % busy, the busiest pipe relative to its rate.  RT_DEQ_MODE picks per half-word: bit 0 = upper half by magic,
-// bit 1 = lower half by magic.  Measured on config 2 (profiles/r2_deq_ab.txt): mode 0 (all I2F) 5880 Mrays/s, mode 1
-// 5746, mode 2 5787, mode 3 5580 — the kernel is bound by issue slots, not by the XU pipe: the second instruction per
-// plane costs more than the slow pipe.  Default 0.
-#ifndef RT_DEQ_MODE
-#define RT_DEQ_MODE 0
-#endif
-__device__ __forceinline__ float q_lo(uint32_t w) {
-#if RT_DEQ_MODE & 2
-    return __uint_as_float(__byte_perm(w, 0x4B000000u, 0x7610)) - 8388608.0f;
-#else
-    return (float)(uint16_t)(w & 0xffffu);
-#endif
-}
-__device__ __forceinline__ float q_hi(uint32_t w) {
-#if RT_DEQ_MODE & 1
-    return __uint_as_float(__byte_perm(w, 0x4B000000u, 0x7632)) - 8388608.0f;
-#else
-    return (float)(uint16_t)(w >> 16);
-#endif
-}
+// exact uint16 -> float with I2F.U16: one instruction that reads the half register directly, but on the XU pipe,
+// 16 lanes / clk / SM (tools/microbench.cu: 4.5 T/s against 17.8 T/s FFMA instructions).  A 4-wide visit converts 24
+// planes; ncu round 2 had XU 54 % busy, the busiest pipe relative to its rate.  Splicing the 16 bits into the mantissa
+// of 2^23 and subtracting 2^23 moves the work to the ALU and FMA pipes, but costs a second instruction per plane, and
+// the kernel is bound by issue slots: that byte-permute variant measured slower for either half and for both
+// (config 2, 5580-5787 vs 5880 Mrays/s, profiles/r2_deq_ab.txt).
+__device__ __forceinline__ float q_lo(uint32_t w) { return (float)(uint16_t)(w & 0xffffu); }
+__device__ __forceinline__ float q_hi(uint32_t w) { return (float)(uint16_t)(w >> 16); }
 
 // The ray in grid coordinates: per-axis scaling of origin and direction leaves t unchanged.
 struct GridRay {
@@ -180,11 +154,11 @@ struct TriGeom {
 };
 __device__ __forceinline__ TriGeom load_tri(const SceneView& sc, int32_t s) {
     float g[8];
-    asm volatile("ld.global.nc" RT_TRI_HINT ".v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+    asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                  : "=f"(g[0]), "=f"(g[1]), "=f"(g[2]), "=f"(g[3]), "=f"(g[4]), "=f"(g[5]), "=f"(g[6]), "=f"(g[7])
                  : "l"(sc.tri_geom + 4 * s));
     float4 h;
-    asm volatile("ld.global.nc" RT_TRI_HINT ".v4.f32 {%0,%1,%2,%3}, [%4];"
+    asm volatile("ld.global.nc.v4.f32 {%0,%1,%2,%3}, [%4];"
                  : "=f"(h.x), "=f"(h.y), "=f"(h.z), "=f"(h.w)
                  : "l"(sc.tri_geom + 4 * s + 2));
     TriGeom t;

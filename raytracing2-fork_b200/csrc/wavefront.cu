@@ -267,36 +267,22 @@ __global__ void __launch_bounds__(kBlock) k_raygen(const __grid_constant__ Frame
 // The closest-hit rule (min dst, then lowest original index) makes the result independent of the
 // order in which lanes, nodes and triangles are visited, so the restructuring changes no bit.
 constexpr int kExtBlock = 128;
-// Software prefetch of the streaming ray records.  Without chunked claims (RT_EXT_CLAIM = 0) every lane asks, at a
-// refill, for the record a lane of this grid will claim about one refill generation later: config 2, 5859 vs 5806
-// Mrays/s (+0.9 %; profiles/r2_prefetch_ab.txt).  With chunked claims the warp knows its next records exactly:
-// 1 = the head of the private range into L2 at every refill, 3 = the same into L1, 2 = the whole chunk that some warp
-// will claim one generation ahead (it is evicted again before it is used often enough to cost 8 B of DRAM traffic per
-// segment: ncu, profiles/r2_traffic_*.csv of the v20 capture), 0 = none.
-#ifndef RT_EXT_PREFETCH
-#define RT_EXT_PREFETCH 1
-#endif
+constexpr int kExtMinBlocks = 9;  // 56 registers: nine resident blocks per SM (ten at 48 registers measured 0.8 % slower, eight slower too)
+// Rays claimed from the queue per atomicAdd on the shared cursor.  Round 1 took one atomic per refill.
+constexpr uint32_t kExtClaim = 128;
+// Software prefetch of the streaming ray records.  With chunked claims the warp knows its next records exactly, and
+// at every refill it prefetches the head of its private range into L2.  Measured and not kept: the same into L1, the
+// whole chunk that some warp will claim one generation ahead (it is evicted again before it is used often enough to
+// cost 8 B of DRAM traffic per segment: ncu, profiles/r2_traffic_*.csv of the v20 capture), and no prefetch.  Before
+// chunked claims, prefetching the record a lane would claim one refill generation later gave
+// config 2 5859 vs 5806 Mrays/s (+0.9 %; profiles/r2_prefetch_ab.txt).
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-#ifndef RT_EXT_TMAX
-#define RT_EXT_TMAX 1   // the triangle test leaves before the barycentrics when dst > best
-#endif
-#ifndef RT_EXT_LAZY_ORIG
-#define RT_EXT_LAZY_ORIG 1
-#endif
-// Rays claimed from the queue per atomicAdd on the shared cursor (0 = one atomic per refill, round 1's scheme).
-#ifndef RT_EXT_CLAIM
-#define RT_EXT_CLAIM 128
-#endif
-#ifndef RT_EXT_MIN_BLOCKS
-#define RT_EXT_MIN_BLOCKS 9   // 56 registers: nine resident blocks per SM (ten at 48 registers measured 0.8 % slower, eight slower too)
-#endif
 constexpr int32_t kPop = (int32_t)0x80000000;       // lane state: take the next subtree from the stack
 constexpr int32_t kIdle = (int32_t)0x80000001;      // lane state: no ray
-struct ExtendTune {
-    int leafVote;  // leaf step when >= this many lanes wait at a leaf
-    int refill;    // refill when >= this many lanes are idle
-    int nodeSteps; // node steps per vote
-};
+// Warp-vote thresholds: a leaf step when >= kLeafVote lanes wait at a leaf, a refill when >= kRefill lanes are idle.
+// Refill 4 / 6 / 12 and leaf vote 12 / 16 measured 0.2-1.7 % slower (DESIGN.md section 5).
+constexpr int kLeafVote = 14;
+constexpr int kRefill = 8;
 
 // One node step for a lane at an inner node: two slab tests, then a branch-free choice of the next
 // state (near child / push far child / pop).  v2's if/else ladder here ran at 3-8 active lanes
@@ -310,10 +296,7 @@ struct RayRegs {
 // [level][thread], so a warp-wide push or pop is conflict-free (one bank pair per lane) whatever
 // the lanes' depths are; in local memory the same access scatters over up to 32 lines and costs up
 // to 32 L1TEX wavefronts.  Deeper entries (rare: most rays keep fewer than 16 pending nodes) overflow to local memory.
-#ifndef RT_SH_STACK
-#define RT_SH_STACK 16
-#endif
-constexpr int kShStack = RT_SH_STACK;
+constexpr int kShStack = 16;
 struct Stack {
     int2* sh;         // &shared[0][threadIdx.x]; stride kExtBlock
     int32_t* ovNode;  // local overflow
@@ -362,21 +345,12 @@ __device__ __forceinline__ void node_step(const SceneView& sc, const RayRegs& r,
 // The same step over a 4-wide node (64 bytes, two 256-bit loads): four slab tests, a 5-comparator sorting network
 // on (entry distance, child) with missed children at +inf, the nearest child becomes the lane's node and the other
 // hit children are pushed farthest first.  Up to three pushes per step.
-// TOP: the first kTopNodes wide nodes (k_collapse4 numbers them level by level, so these are the root and the three
-// levels below it: 1 + 4 + 16 + 64) are read from the block's shared-memory copy instead of L1 / L2.
-constexpr int kTopNodes = 85;
-template <bool DEEP, bool WIDEN, bool TOP>
-__device__ __forceinline__ void node_step4(const SceneView& sc, const uint4* __restrict__ sTop, const RayRegs& r,
-                                           int32_t& node, int& sp, Stack& st) {
+// (Staging the root and the three levels below it in shared memory measured -3 %: those nodes are L1 hits already.)
+template <bool DEEP, bool WIDEN>
+__device__ __forceinline__ void node_step4(const SceneView& sc, const RayRegs& r, int32_t& node, int& sp, Stack& st) {
     uint32_t a[8], b[8];
-    if (TOP && node < kTopNodes) {
-        const uint4 q0 = sTop[4 * node + 0], q1 = sTop[4 * node + 1], q2 = sTop[4 * node + 2], q3 = sTop[4 * node + 3];
-        a[0] = q0.x; a[1] = q0.y; a[2] = q0.z; a[3] = q0.w; a[4] = q1.x; a[5] = q1.y; a[6] = q1.z; a[7] = q1.w;
-        b[0] = q2.x; b[1] = q2.y; b[2] = q2.z; b[3] = q2.w; b[4] = q3.x; b[5] = q3.y; b[6] = q3.z; b[7] = q3.w;
-    } else {
-        ldg256u(sc.nodes4 + 4 * node, a);
-        ldg256u(sc.nodes4 + 4 * node + 2, b);
-    }
+    ldg256u(sc.nodes4 + 4 * node, a);
+    ldg256u(sc.nodes4 + 4 * node + 2, b);
     float t[4];
     int32_t c[4] = {(int32_t)b[4], (int32_t)b[5], (int32_t)b[6], (int32_t)b[7]};
     t[0] = slab1<WIDEN>(a[0], a[1], a[2], r.g, r.bestT);
@@ -407,12 +381,16 @@ __device__ __forceinline__ bool is_leaf_code(int32_t x) { return x < 0 && (uint3
 // SPEC = speculative traversal (Aila & Laine's "postponed leaf"): a lane that reaches a leaf parks it in
 // `post` and keeps descending; it only has to wait for a leaf step when it reaches a SECOND leaf (or runs
 // out of nodes).  Node steps then run with more lanes, leaf steps test up to two leaves per lane; the price
-// is a stale bestT while a leaf is parked (a few more node visits).  Selected at run time (RT_EXT_SPEC).
-template <bool COUNT, bool SPEC, bool WIDE, bool WIDEN, bool TOP>
-__global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const __grid_constant__ SceneView sc, PathArrays cur,
+// is a stale bestT while a leaf is parked (a few more node visits).  How far a lane runs ahead of its parked leaf
+// depends on the other lanes of its warp, so the instrumented variants (COUNT) walk without it: their node-visit
+// and triangle-test counts are those of each ray's own sequential walk.
+template <bool COUNT, bool WIDE, bool WIDEN>
+__global__ void __launch_bounds__(kExtBlock, kExtMinBlocks) k_extend(const __grid_constant__ SceneView sc, PathArrays cur,
                                                       float4* __restrict__ hit, const uint32_t* __restrict__ count,
-                                                      uint32_t* __restrict__ cursor, ExtendTune tune,
+                                                      uint32_t* __restrict__ cursor,
                                                       unsigned long long* __restrict__ stats) {
+    constexpr bool SPEC = !COUNT;
+    constexpr int kNodeSteps = WIDE ? 2 : 4;  // node steps per vote (3 on the 4-wide tree, 3 / 6 on the binary one: slower)
     const uint32_t n = *count;
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&stats[0], (unsigned long long)n);
     const uint32_t lane = threadIdx.x & 31u;
@@ -421,17 +399,9 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
     const float kWiden = WIDEN ? kWidenFar : 1.0f;  // x * 1.0f folds away
 
     __shared__ int2 shStack[kShStack][kExtBlock];
-#if RT_EXT_CLAIM > 0
     __shared__ uint32_t sClaim[kExtBlock / 32][4];  // per warp: next, end of its private range; queue exhausted
     if ((threadIdx.x & 31u) == 0u) { sClaim[threadIdx.x >> 5][0] = 0u; sClaim[threadIdx.x >> 5][1] = 0u; sClaim[threadIdx.x >> 5][2] = 0u; }
     __syncwarp();
-#endif
-    __shared__ uint4 sTop[TOP ? 4 * kTopNodes : 1];
-    if (TOP) {
-        const int have = min(4 * kTopNodes, 4 * sc.num_nodes4);
-        for (int k = threadIdx.x; k < have; k += kExtBlock) sTop[k] = __ldg(&sc.nodes4[k]);
-        __syncthreads();
-    }
     int32_t ovNode[kStackSize - kShStack];
     float ovT[kStackSize - kShStack];
     Stack st{&shStack[0][threadIdx.x], ovNode, ovT};
@@ -441,7 +411,7 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
     r.o = v3(0, 0, 0); r.d = v3(0, 0, 1); r.bestT = kMissT;
     r.g.ox = r.g.oy = r.g.oz = r.g.ix = r.g.iy = r.g.iz = r.g.nx = r.g.ny = r.g.nz = 0.0f;
     float bestU = 0, bestV = 0;
-    int32_t bestSlot = -1, bestOrig = 0x7fffffff;
+    int32_t bestSlot = -1;
     int32_t node = kIdle;
     int32_t post = kNoLeaf;
     int sp = 0;
@@ -457,8 +427,8 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
         const TriGeom tg = load_tri(sc, s);
         if (COUNT) tests++;
         float dst, u, v;
-        if (ray_triangle(r.o, r.d, tg.a, tg.e0, tg.e1, tg.N, dst, u, v, RT_EXT_TMAX ? r.bestT : 3.4e38f)) {
-#if RT_EXT_LAZY_ORIG
+        // the test leaves before the barycentrics when dst > best
+        if (ray_triangle(r.o, r.d, tg.a, tg.e0, tg.e1, tg.N, dst, u, v, r.bestT)) {
             // the original indices are needed only to break an exact tie in dst: fetch them then, not for every
             // candidate (the dependent 4-byte gather was 3.4 % of k_extend's stall samples)
             if (dst <= r.bestT && dst < kMissT) {
@@ -468,14 +438,6 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
                     r.bestT = dst; bestU = u; bestV = v; bestSlot = s;
                 }
             }
-#else
-            if (dst <= r.bestT && dst < kMissT) {
-                const int32_t orig = __ldg(&sc.tri_orig[s]);
-                if (dst < r.bestT || orig < bestOrig) {
-                    r.bestT = dst; bestU = u; bestV = v; bestSlot = s; bestOrig = orig;
-                }
-            }
-#endif
         }
     };
     auto test_leaf = [&](int32_t code) {
@@ -518,14 +480,12 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
         }
         if (node >= 0) {
             if (COUNT) visits++;
-            if (WIDE) node_step4<DEEP, WIDEN, TOP>(sc, sTop, r, node, sp, st);
+            if (WIDE) node_step4<DEEP, WIDEN>(sc, r, node, sp, st);
             else node_step<DEEP, WIDEN>(sc, r, node, sp, st);
             if (SPEC) {
                 const bool park = is_leaf_code(node) & (post == kNoLeaf);
                 post = park ? node : post;
                 node = park ? kPop : node;
-            } else {
-                postpone();
             }
         }
     };
@@ -547,9 +507,8 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
         }
         // ---- refill idle lanes from the queue
         uint32_t idle = __ballot_sync(FULL, node == kIdle);
-#if RT_EXT_CLAIM > 0
-        if (!exhausted && ((int)__popc(idle) >= tune.refill || idle == FULL)) {
-            // The warp owns a private range [next, end) of the queue, claimed RT_EXT_CLAIM rays at a time: one atomic on
+        if (!exhausted && ((int)__popc(idle) >= kRefill || idle == FULL)) {
+            // The warp owns a private range [next, end) of the queue, claimed kExtClaim rays at a time: one atomic on
             // the shared cursor per chunk instead of one per refill, and a refill out of the private range waits for no
             // atomic at all.  The leftover of a range is handed out before the fresh chunk, so no ray is skipped.
             uint32_t* const cl = sClaim[threadIdx.x >> 5];
@@ -560,14 +519,10 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
             uint32_t fbase = 0, fend = 0;
             if (fresh) {
                 const int leader = __ffs(idle) - 1;
-                if ((int)lane == leader) fbase = atomicAdd(cursor, (uint32_t)RT_EXT_CLAIM);
+                if ((int)lane == leader) fbase = atomicAdd(cursor, kExtClaim);
                 fbase = __shfl_sync(FULL, fbase, leader);
                 fbase = min(fbase, n);
-                fend = min(fbase + (uint32_t)RT_EXT_CLAIM, n);
-                if (RT_EXT_PREFETCH == 2) {  // the chunk a warp of this grid will claim about one generation from now
-                    const uint32_t ahead = fbase + gridDim.x * (kExtBlock / 32) * (uint32_t)RT_EXT_CLAIM + 8u * (lane & 15u);
-                    if (ahead < n && 8u * (lane & 15u) < (uint32_t)RT_EXT_CLAIM) prefetch_l2(lane < 16u ? &cur.od0[ahead] : &cur.od1[ahead]);
-                }
+                fend = min(fbase + kExtClaim, n);
             }
             if (node == kIdle) {
                 const uint32_t rank = __popc(idle & ltMask);
@@ -584,7 +539,7 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
                     r.o = v3(a.x, a.y, a.z);
                     r.d = v3(a.w, b.x, b.y);
                     r.g = make_grid_ray(sc, r.o, r.d);
-                    r.bestT = kMissT; bestU = 0.0f; bestV = 0.0f; bestSlot = -1; bestOrig = 0x7fffffff;
+                    r.bestT = kMissT; bestU = 0.0f; bestV = 0.0f; bestSlot = -1;
                     sp = 0;
                     post = kNoLeaf;
                     node = sc.root_is_leaf ? pack_leaf(0, sc.num_tris) : 0;
@@ -600,15 +555,12 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
                 nnext = next + min(want, avail);
                 nend = end;
             }
-            if ((RT_EXT_PREFETCH == 1 || RT_EXT_PREFETCH == 3) && lane < 10u) {
+            if (lane < 10u) {
                 // the records this warp takes at its NEXT refill are known exactly: the head of its private range
                 // (five 128-byte lines of each array cover 32 records wherever the range starts)
                 const uint32_t p = nnext + 8u * (lane < 5u ? lane : lane - 5u);
                 const void* q = lane < 5u ? (const void*)&cur.od0[p] : (const void*)&cur.od1[p];
-                if (p < nend) {
-                    if (RT_EXT_PREFETCH == 3) asm volatile("prefetch.global.L1 [%0];" ::"l"(q));
-                    else prefetch_l2(q);
-                }
+                if (p < nend) prefetch_l2(q);
             }
             __syncwarp();
             if (lane == 0) { cl[0] = nnext; cl[1] = nend; cl[2] = ndone; }
@@ -616,37 +568,6 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
             if (ndone != 0u && nnext == nend) exhausted = true;
             idle = __ballot_sync(FULL, node == kIdle);
         }
-#else
-        if (!exhausted && ((int)__popc(idle) >= tune.refill || idle == FULL)) {
-            uint32_t base = 0;
-            const int leader = __ffs(idle) - 1;
-            const uint32_t want = __popc(idle);
-            if ((int)lane == leader) base = atomicAdd(cursor, want);
-            base = __shfl_sync(FULL, base, leader);
-            if (node == kIdle) {
-                const uint32_t i = base + __popc(idle & ltMask);
-                if (RT_EXT_PREFETCH != 0) {  // the record a lane of this grid will claim about one refill generation from now
-                    const uint32_t ahead = i + gridDim.x * kExtBlock;
-                    if (ahead < n) { prefetch_l2(&cur.od0[ahead]); prefetch_l2(&cur.od1[ahead]); }
-                }
-                if (i < n) {
-                    const float4 a = cur.od0[i];
-                    const float4 b = cur.od1[i];
-                    ray = i;
-                    r.o = v3(a.x, a.y, a.z);
-                    r.d = v3(a.w, b.x, b.y);
-                    r.g = make_grid_ray(sc, r.o, r.d);
-                    r.bestT = kMissT; bestU = 0.0f; bestV = 0.0f; bestSlot = -1; bestOrig = 0x7fffffff;
-                    sp = 0;
-                    post = kNoLeaf;
-                    node = sc.root_is_leaf ? pack_leaf(0, sc.num_tris) : 0;
-                    postpone();
-                }
-            }
-            if (base + want >= n) exhausted = true;
-            idle = __ballot_sync(FULL, node == kIdle);
-        }
-#endif
         if (idle == FULL) {
             if (exhausted) break;
             continue;
@@ -655,7 +576,7 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
         const bool parked = is_leaf_code(node) || node == kDrain;
         const uint32_t parkedM = __ballot_sync(FULL, parked);
         const uint32_t nodeM = __ballot_sync(FULL, node >= 0 || (SPEC && node == kPop));
-        if ((int)__popc(parkedM) >= tune.leafVote || nodeM == 0u) {
+        if ((int)__popc(parkedM) >= kLeafVote || nodeM == 0u) {
             if (SPEC) {
                 if (post != kNoLeaf) {
                     test_leaf(post);
@@ -670,14 +591,14 @@ __global__ void __launch_bounds__(kExtBlock, RT_EXT_MIN_BLOCKS) k_extend(const _
         } else {
             // several node steps per vote amortise the voting overhead.  When no lane can reach the end of the
             // shared part of its stack within this round, the loop without any overflow code runs.
-            const bool deep = __any_sync(FULL, sp + (WIDE ? 3 : 1) * tune.nodeSteps >= kShStack);
+            const bool deep = __any_sync(FULL, sp + (WIDE ? 3 : 1) * kNodeSteps >= kShStack);
             const float bestW = r.bestT * kWiden;
             if (!deep) {
 #pragma unroll 1
-                for (int k = 0; k < tune.nodeSteps; k++) node_iter_impl(std::false_type{}, bestW);
+                for (int k = 0; k < kNodeSteps; k++) node_iter_impl(std::false_type{}, bestW);
             } else {
 #pragma unroll 1
-                for (int k = 0; k < tune.nodeSteps; k++) node_iter_impl(std::true_type{}, bestW);
+                for (int k = 0; k < kNodeSteps; k++) node_iter_impl(std::true_type{}, bestW);
             }
         }
     }
@@ -856,37 +777,42 @@ __device__ __forceinline__ BounceRandoms bounce_randoms(Rng<1>& rng, bool needDi
 // Also measured and removed (profiles/r2_final_ab.txt): gathering the NEXT window's hit-triangle record into L1 / L2
 // while this one is shaded (config 2 6039 / 6029 vs 6049-6059, config 4 +0.9 %), three resident blocks at 80 registers
 // without spills (6018), a smaller shade grid (32 / 16 blocks per SM: 6030 / 5981).
-#ifndef RT_SHADE_MIN_BLOCKS
-#define RT_SHADE_MIN_BLOCKS 4   // 64 registers; 5 blocks (48 registers, 358 B of spills) -15 %, 6 blocks -16 % (profiles/r2_leafmerge_shadeocc_ab.txt)
-#endif
-template <int MODE, int DEFER>
-__global__ void __launch_bounds__(kBlock, RT_SHADE_MIN_BLOCKS) k_shade(const __grid_constant__ SceneView sc,
+constexpr int kShadeMinBlocks = 4;  // 64 registers; 5 blocks (48 registers, 358 B of spills) -15 %, 6 blocks -16 % (profiles/r2_leafmerge_shadeocc_ab.txt)
+// Windows per deferred queue reservation.  Measured on four boxes (profiles/r2_final_ab.txt): config 2, bounce 0
+// deferred, 1 / 2 / 3 / 4 windows 6059-6066 / 6077 / 6115-6128 / 6063 Mrays/s on every box; config 4, every bounce
+// deferred, 1 window 4146 / 4410 / 4540 / 4542 depending on the box (the atomic's latency and rate are the box lottery
+// of DESIGN.md section 6.1), 2 windows 4229 / 4257 / 4515, 3 windows 4449 / 4454 / 4461 on all of them, 4 windows
+// (48 KB of staging per block: too little L1 left) 4179.
+constexpr int kDeferWindows = 3;
+template <int MODE, bool DEFER>
+__global__ void __launch_bounds__(kBlock, kShadeMinBlocks) k_shade(const __grid_constant__ SceneView sc,
                                                   const __grid_constant__ FrameParams fp, PathArrays cur,
                                                   PathArrays next, const float4* __restrict__ hit,
                                                   float4* __restrict__ contrib, uint32_t* __restrict__ pix_rng,
                                                   const uint32_t* __restrict__ countIn,
                                                   uint32_t* __restrict__ countOut, int bounce) {
     __shared__ CoopSlot sCoop[kBlock / 32][kCoopOwners];  // stage 2 of bounce_randoms: keys handed to the warp
-    // DEFER = W > 0: the survivors of W consecutive windows wait in shared memory, every lane in its own slot, while
-    // the warp's ONE queue reservation for them is in flight
-    extern __shared__ float4 sStageDyn[];  // [DEFER][3][kBlock], sized at launch (12 KB per window)
+    // DEFER: the survivors of kDeferWindows consecutive windows wait in shared memory, every lane in its own slot,
+    // while the warp's ONE queue reservation for them is in flight
+    constexpr int kWin = DEFER ? kDeferWindows : 1;
+    extern __shared__ float4 sStageDyn[];  // [kDeferWindows][3][kBlock], sized at launch (12 KB per window)
 #define sStage(k, c) sStageDyn[((k) * 3 + (c)) * kBlock + threadIdx.x]
     const uint32_t n = *countIn;
     const uint32_t lane = threadIdx.x & 31u;
     constexpr uint32_t FULL = 0xffffffffu;
-    uint32_t pend[DEFER ? DEFER : 1];  // survivor masks of the windows of the batch being staged / in flight
+    uint32_t pend[kWin];  // survivor masks of the windows of the batch being staged / in flight
 #pragma unroll
-    for (int k = 0; k < (DEFER ? DEFER : 1); k++) pend[k] = 0u;
+    for (int k = 0; k < kWin; k++) pend[k] = 0u;
     uint32_t pendRaw = 0u, phase = 0u;  // lane 0: the atomicAdd result; which window of the batch comes next
     // the batch in flight goes to the queue: window k of it behind the survivors of windows 0 .. k-1
     auto flush = [&]() {
         uint32_t any = 0u;
 #pragma unroll
-        for (int k = 0; k < (DEFER ? DEFER : 1); k++) any |= pend[k];
+        for (int k = 0; k < kWin; k++) any |= pend[k];
         if (any == 0u) return;
         uint32_t at = __shfl_sync(FULL, pendRaw, 0);
 #pragma unroll
-        for (int k = 0; k < (DEFER ? DEFER : 1); k++) {
+        for (int k = 0; k < kWin; k++) {
             if ((pend[k] >> lane) & 1u) {
                 const uint32_t pos = at + __popc(pend[k] & ((1u << lane) - 1u));
                 next.od0[pos] = sStage(k, 0);
@@ -899,7 +825,7 @@ __global__ void __launch_bounds__(kBlock, RT_SHADE_MIN_BLOCKS) k_shade(const __g
     auto reserve = [&]() {
         uint32_t total = 0u;
 #pragma unroll
-        for (int k = 0; k < (DEFER ? DEFER : 1); k++) total += __popc(pend[k]);
+        for (int k = 0; k < kWin; k++) total += __popc(pend[k]);
         if (total != 0u && lane == 0u) pendRaw = atomicAdd(countOut, total);
     };
     for (uint32_t base = blockIdx.x * kBlock; base < n; base += gridDim.x * kBlock) {
@@ -1035,19 +961,19 @@ __global__ void __launch_bounds__(kBlock, RT_SHADE_MIN_BLOCKS) k_shade(const __g
         }
         // compaction: the survivors of this warp take consecutive places in the next queue
         const uint32_t mask = __ballot_sync(FULL, alive);
-        if (DEFER > 0) {
+        if (DEFER) {
             // Deferred append.  The warp's atomicAdd on the queue counter takes microseconds to return, and the 4.2 M of
             // them per 133 M-path launch all hit one address (ncu, v19: 41.6 % of k_shade's stall samples at bounce 0
             // of config 2 and 44 % at every bounce of config 4 sat on the shuffle that broadcasts the result).  So the
-            // survivors of DEFER consecutive windows share ONE reservation, issued when the last of them is staged,
+            // survivors of kDeferWindows consecutive windows share ONE reservation, issued when the last of them is staged,
             // and are written to the queue at the end of the window after that — a whole iteration later.
             if (phase == 0u) {
                 flush();
 #pragma unroll
-                for (int k = 0; k < DEFER; k++) pend[k] = 0u;
+                for (int k = 0; k < kWin; k++) pend[k] = 0u;
             }
 #pragma unroll
-            for (int k = 0; k < DEFER; k++)
+            for (int k = 0; k < kWin; k++)
                 if ((uint32_t)k == phase) pend[k] = mask;
             if (alive) {
                 sStage(phase, 0) = make_float4(o.x, o.y, o.z, d.x);
@@ -1055,7 +981,7 @@ __global__ void __launch_bounds__(kBlock, RT_SHADE_MIN_BLOCKS) k_shade(const __g
                 sStage(phase, 2) = make_float4(rayColor.z, __int_as_float(slotId), __uint_as_float(carry),
                                                __uint_as_float(flags));
             }
-            phase = phase + 1u == (uint32_t)DEFER ? 0u : phase + 1u;
+            phase = phase + 1u == (uint32_t)kWin ? 0u : phase + 1u;
             if (phase == 0u) reserve();
         } else {
             uint32_t basePos = 0;
@@ -1073,7 +999,7 @@ __global__ void __launch_bounds__(kBlock, RT_SHADE_MIN_BLOCKS) k_shade(const __g
             }
         }
     }
-    if (DEFER > 0) {
+    if (DEFER) {
         if (phase != 0u) reserve();  // an incomplete last batch has no reservation yet
         flush();
     }
@@ -1365,17 +1291,15 @@ struct Timed {
     }
 };
 
-int wf_extend_blocks_per_sm(bool instrument, bool wide, bool top) {
+int wf_extend_blocks_per_sm(bool instrument, bool wide) {
     int nb = 0;
     cudaError_t e;
-    if (wide && top)
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, true, true, false, true>, kExtBlock, 0);
-    else if (wide)
-        e = instrument ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<true, false, true, true, false>, kExtBlock, 0)
-                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, true, true, false, false>, kExtBlock, 0);
+    if (wide)
+        e = instrument ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<true, true, true>, kExtBlock, 0)
+                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, true, false>, kExtBlock, 0);
     else
-        e = instrument ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<true, false, false, true, false>, kExtBlock, 0)
-                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, true, false, false, false>, kExtBlock, 0);
+        e = instrument ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<true, false, true>, kExtBlock, 0)
+                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, false, false>, kExtBlock, 0);
     return e == cudaSuccess && nb > 0 ? nb : 4;
 }
 
@@ -1384,18 +1308,17 @@ int wf_extend_blocks_per_sm(bool instrument, bool wide, bool top) {
 static void launch_extend(const Launcher& L, const SceneView& sc, const PathArrays& rays, float4* hit,
                           const uint32_t* count, uint32_t* cursor, bool widen, unsigned long long* stats) {
     const bool wide = sc.nodes4 != nullptr;
-    ExtendTune tune{L.leaf_vote, L.refill, wide ? L.node_steps_wide : L.node_steps};
     const int grid = wide ? L.extend_grid_wide : L.extend_grid;
     cudaStream_t st = L.st;
-#define RT_EXT(C, S, W, WD, T) k_extend<C, S, W, WD, T><<<grid, kExtBlock, 0, st>>>(sc, rays, hit, count, cursor, tune, stats)
+#define RT_EXT(C, W, WD) k_extend<C, W, WD><<<grid, kExtBlock, 0, st>>>(sc, rays, hit, count, cursor, stats)
     if (wide) {
-        if (L.instrument) RT_EXT(true, false, true, true, false);
-        else if (L.top_smem) { if (widen) RT_EXT(false, true, true, true, true); else RT_EXT(false, true, true, false, true); }
-        else { if (widen) RT_EXT(false, true, true, true, false); else RT_EXT(false, true, true, false, false); }
+        if (L.instrument) RT_EXT(true, true, true);
+        else if (widen) RT_EXT(false, true, true);
+        else RT_EXT(false, true, false);
     } else {
-        if (L.instrument) RT_EXT(true, false, false, true, false);
-        else if (!L.speculative) RT_EXT(false, false, false, true, false);
-        else { if (widen) RT_EXT(false, true, false, true, false); else RT_EXT(false, true, false, false, false); }
+        if (L.instrument) RT_EXT(true, false, true);
+        else if (widen) RT_EXT(false, false, true);
+        else RT_EXT(false, false, false);
     }
 #undef RT_EXT
     (*L.kernel_launches)++;
@@ -1435,41 +1358,25 @@ cudaError_t wf_render_batch(const Launcher& L, const SceneView& sc, const WaveBu
         {
             Timed t(L, 0);
             // camera rays may start far outside the scene; every later segment starts on a surface of it
-            launch_extend(L, sc, a, wb.hit, wb.counts + bounce, cursors + bounce, bounce == 0 ? L.widen_primary : L.widen_always, wb.stats);
+            launch_extend(L, sc, a, wb.hit, wb.counts + bounce, cursors + bounce, bounce == 0 && L.widen_primary, wb.stats);
         }
         {
             Timed t(L, 1);
-            // Deferred append (see k_shade): 0 never, 1 at bounce 0 only, 2 at every bounce, 3 (default) at bounce 0 and,
-            // when the scene has no textures, at every bounce.  Measured on B200 (profiles/r2_final_ab.txt): bounce 0 is
-            // latency-bound everywhere (config 2: +1.5 % from deferring it alone); the later bounces of the textured
-            // config-2 scene are issue-bound (66 % issue-active, 17.8 lanes per instruction) and LOSE 0.8-2.4 % to the
-            // staging, those of the untextured 10 M-triangle scene wait on the atomic like bounce 0 does (34 %
-            // issue-active, 44 % of the stall samples) and gain 3.3-9.4 % depending on the box.
-            const bool defer = L.shade_defer == 2 || (L.shade_defer == 1 && bounce == 0) ||
-                               (L.shade_defer >= 3 && (bounce < L.shade_defer_bounces || fp.u.numTextures <= 0));
-            // Windows per reservation: 3 (RT_SHADE_DEFER_BATCH at bounce 0, RT_SHADE_DEFER_BATCH_LATER afterwards).
-            // Measured on four boxes (profiles/r2_final_ab.txt): config 2, bounce 0 deferred, 1 / 2 / 3 / 4 windows
-            // 6059-6066 / 6077 / 6115-6128 / 6063 Mrays/s on every box; config 4, every bounce deferred, 1 window
-            // 4146 / 4410 / 4540 / 4542 depending on the box (the atomic's latency and rate are the box lottery of
-            // DESIGN.md section 6.1), 2 windows 4229 / 4257 / 4515, 3 windows 4449 / 4454 / 4461 on all of them, 4
-            // windows (48 KB of staging per block: too little L1 left) 4179.
-            const int dmode = defer ? std::max(1, std::min(3, bounce == 0 ? L.shade_defer_batch : L.shade_defer_batch_later)) : 0;
-            const size_t stage_bytes = (size_t)dmode * 3 * kBlock * sizeof(float4);
+            // Deferred append (see k_shade) at bounce 0 and, when the scene has no textures, at every bounce.  Measured
+            // on B200 (profiles/r2_final_ab.txt): bounce 0 is latency-bound everywhere (config 2: +1.5 % from deferring
+            // it alone); the later bounces of the textured config-2 scene are issue-bound (66 % issue-active, 17.8 lanes
+            // per instruction) and LOSE 0.8-2.4 % to the staging, those of the untextured 10 M-triangle scene wait on
+            // the atomic like bounce 0 does (34 % issue-active, 44 % of the stall samples) and gain 3.3-9.4 % depending
+            // on the box.
+            const bool defer = bounce == 0 || fp.u.numTextures <= 0;
+            const size_t stage_bytes = defer ? (size_t)kDeferWindows * 3 * kBlock * sizeof(float4) : 0;
 #define RT_SHADE(M, D) k_shade<M, D><<<grid, kBlock, stage_bytes, L.st>>>(sc, fp, a, b, wb.hit, wb.contrib, wb.pix_rng, wb.counts + bounce, \
                                                                         wb.counts + bounce + 1, bounce)
-#define RT_SHADE_M(M)                          \
-    switch (dmode) {                           \
-        case 0: RT_SHADE(M, 0); break;         \
-        case 1: RT_SHADE(M, 1); break;         \
-        case 2: RT_SHADE(M, 2); break;         \
-        default: RT_SHADE(M, 3); break;        \
-    }
             if (L.rng_mode == RT_RNG_REF_PCG) {
-                RT_SHADE_M(0)
+                if (defer) RT_SHADE(0, true); else RT_SHADE(0, false);
             } else {
-                RT_SHADE_M(1)
+                if (defer) RT_SHADE(1, true); else RT_SHADE(1, false);
             }
-#undef RT_SHADE_M
 #undef RT_SHADE
             (*L.kernel_launches)++;
         }

@@ -656,16 +656,14 @@ def test_real_asset_robot_if_generated():
 
 
 # ------------------------------------------------------------------------------------------------ round 2
-@pytest.mark.parametrize("env", [{"RT_EXT_TOP": "1"}, {"RT_HOOKS": "thread"}, {"RT_BVH_WIDTH": "2"}, {"RT_MAX_PATHS_MI": "1"},
-                                 {"RT_BVH_BUILDER": "lbvh"}, {"RT_BVH_BUILDER": "lbvh", "RT_BVH_WIDTH": "2"},
-                                 {"RT_EXT_WIDEN": "1"}, {"RT_SHADE_DEFER": "0"}, {"RT_SHADE_DEFER": "2"},
-                                 {"RT_SHADE_DEFER": "2", "RT_SHADE_DEFER_BATCH": "1", "RT_SHADE_DEFER_BATCH_LATER": "3"}])
+@pytest.mark.parametrize("env", [{"RT_HOOKS": "thread"}, {"RT_BVH_WIDTH": "2"}, {"RT_MAX_PATHS_MI": "1"},
+                                 {"RT_BVH_BUILDER": "lbvh"}, {"RT_BVH_BUILDER": "lbvh", "RT_BVH_WIDTH": "2"}])
 @pytest.mark.parametrize("rng_mode", [rt.RNG_REF_PCG, rt.RNG_PHILOX])
 def test_kernel_variants_change_no_bit(monkeypatch, env, rng_mode):
-    """The shared-memory top of the tree, the per-thread hooks, the binary tree, the Karras builder, the always-widened
-    slab test, k_shade's deferred queue append (never / at every bounce with 3 + 2 or 1 + 3 windows per reservation; the
-    default defers bounce 0) and a tiny path budget only reorder or re-route work: frame, first-hit map and random rays must equal
-    the oracle bit for bit under every switch (the defaults are covered by every other test)."""
+    """The per-thread hooks, the binary tree, the Karras builder and a tiny path budget only reorder or re-route work:
+    frame, first-hit map and random rays must equal the oracle bit for bit under every switch (the defaults are covered
+    by every other test).  Both append policies of k_shade run in every case: the material zoo has no textures, so every
+    bounce defers its queue append; the textured mirror scene defers bounce 0 and appends the later bounces at once."""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     zoo = scenes.material_zoo()
@@ -823,23 +821,23 @@ def test_ray_counts_around_the_claim_size(sphere_box):
     be.close()
 
 
-@pytest.mark.parametrize("env", [{"RT_SHADE_DEFER": "2"},
-                                 {"RT_SHADE_DEFER": "2", "RT_SHADE_DEFER_BATCH": "2", "RT_SHADE_DEFER_BATCH_LATER": "1"},
-                                 {"RT_SHADE_DEFER": "0"}])
-def test_deferred_append_over_many_windows_per_block(monkeypatch, classic, env):
+@pytest.mark.parametrize("scene_name", ["classic", "sphere_box"])
+@pytest.mark.parametrize("rng_mode", [rt.RNG_REF_PCG, rt.RNG_PHILOX])
+def test_deferred_append_over_many_windows_per_block(monkeypatch, request, scene_name, rng_mode):
     """k_shade's deferred append keeps up to three windows of survivors in shared memory per warp and reserves their
     queue places with one atomic; the batches only cycle when a block shades several windows.  A one-block-per-SM shade
     grid over a 448x448 x 2 spp frame gives every block five to eleven windows per bounce (full batches, a ragged last one, the
     final flush; in RT_RNG_REF_PCG mode a wave holds one sample per pixel, hence the 448x448 image): the frame must
-    equal the oracle's bit for bit, in both RNG modes."""
-    scene, orc = classic
+    equal the oracle's bit for bit.  The classic box has no textures, so every bounce defers its append; the textured
+    sphere defers bounce 0 and appends the later bounces at once."""
+    scene, orc = request.getfixturevalue(scene_name)
     monkeypatch.setenv("RT_SHADE_BLOCKS_PER_SM", "1")
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
-    cam = rt.make_camera(448, 448, (0.0, 0.0, 15.5))
+    if scene_name == "classic":
+        cam = rt.make_camera(448, 448, (0.0, 0.0, 15.5))
+    else:
+        cam = rt.camera_for_box(scene, 448, 448)
     u = rt.screenshot_uniforms(scene, cam, spp=2, max_bounce=8, env_light=False)
-    for rng_mode in (rt.RNG_REF_PCG, rt.RNG_PHILOX):
-        be = backend(scene, rng_mode=rng_mode)
-        be.render_frame(u)
-        assert_image_equal(be.read_frame(), orc.render_frame(u, rng_mode=rng_mode), f"deferred append {env}")
-        be.close()
+    be = backend(scene, rng_mode=rng_mode)
+    be.render_frame(u)
+    assert_image_equal(be.read_frame(), orc.render_frame(u, rng_mode=rng_mode), f"deferred append, {scene_name}")
+    be.close()
