@@ -262,6 +262,26 @@ int rt_first_hit(rt_ctx* ctx, const rt_uniforms* uniforms, int32_t mode, int32_t
 int rt_trace_rays(rt_ctx* ctx, const float* origins, const float* dirs, int64_t count,
                   int32_t* tri_id, float* dst, float* bary_u, float* bary_v);
 
+/* ---------------------------------------------------------------- ray queries on device memory
+ * Ray queries on DEVICE memory, asynchronous on the ctx stream (rt_set_stream): no host synchronisation and no device
+ * allocation once the scene is built.  origins / dirs: count*3 floats; tmax: count floats or NULL (unbounded).
+ * A hit needs 1e-6 < t < min(tmax, 1e38); a NaN, zero or negative tmax never hits.  Every pointer must be device
+ * (or managed) memory of cfg.device, else RT_ERR_INVALID; so are count < 0 and count > 2^30, both rejected before
+ * anything is enqueued.  count == 0 returns RT_OK and launches nothing; an unbuilt scene returns RT_ERR_STATE.
+ * The ray count and work cursor are device words of the ctx, so two queries on one ctx are ordered by the ctx
+ * stream, as every other call is: the caller orders the stream against the producers of the inputs and the consumers
+ * of the outputs (e.g. with events).
+ *
+ * rt_query_closest: the closest hit, exactly what rt_trace_rays reports for the same ray when its distance is below
+ * tmax, and a miss otherwise.  tri_id indexes the array given to rt_scene_set_triangles, exact ties go to the lowest
+ * id; a miss writes -1 / 1e38 / 0 / 0.  Outputs may be NULL (not written); they are written in stream order. */
+int rt_query_closest(rt_ctx* ctx, const float* origins, const float* dirs, const float* tmax, int64_t count,
+                     int32_t* tri_id, float* dst, float* bary_u, float* bary_v);
+/* rt_query_occluded: occluded[i] = 1 if some triangle is hit with t < tmax[i], else 0 (the same as
+ * rt_query_closest's dst < tmax, but the walk stops at the first such triangle).  occluded must not be NULL. */
+int rt_query_occluded(rt_ctx* ctx, const float* origins, const float* dirs, const float* tmax, int64_t count,
+                      uint8_t* occluded);
+
 /* Export the GPU-built BVH: call with nodes == NULL to get sizes.  sorted_tri_ids[slot] = original
  * triangle index stored at that leaf slot. */
 int rt_scene_get_bvh(rt_ctx* ctx, rt_bvh_node* nodes, int64_t* node_count, int32_t* sorted_tri_ids,

@@ -173,7 +173,8 @@ ABI_SYMBOLS = [
     "rt_create", "rt_destroy", "rt_last_error", "rt_version", "rt_set_stream",
     "rt_scene_set_triangles", "rt_scene_set_materials", "rt_scene_set_texture", "rt_scene_build",
     "rt_render_frame", "rt_read_frame_rgba32f", "rt_screenshot", "rt_screenshot_device",
-    "rt_screenshot_fetch", "rt_screenshot_partial", "rt_read_frame_sum", "rt_finalize_sums", "rt_first_hit", "rt_trace_rays", "rt_scene_get_bvh", "rt_get_counters",
+    "rt_screenshot_fetch", "rt_screenshot_partial", "rt_read_frame_sum", "rt_finalize_sums", "rt_first_hit", "rt_trace_rays",
+    "rt_query_closest", "rt_query_occluded", "rt_scene_get_bvh", "rt_get_counters",
     "rt_reset_counters", "rt_comm_unique_id", "rt_comm_init", "rt_split_rows", "rt_split_frames", "rt_plan_batches",
 ]
 
@@ -371,6 +372,8 @@ class Backend:
             self.h = None
             raise BackendError(f"rt_create failed ({rc}): {msg}")
         self.width = self.height = 0
+        self._stream_ptr = 0       # the stream the ctx is bound to (0 = the ctx's own stream, unknown to torch)
+        self._query_stream = None  # its torch view, made by the first ray query
 
     def close(self):
         if getattr(self, "h", None):
@@ -389,6 +392,8 @@ class Backend:
 
     def set_stream(self, cuda_stream_ptr: int):
         self._chk(self.L.rt_set_stream(self.h, C.c_void_p(cuda_stream_ptr)))
+        self._stream_ptr = int(cuda_stream_ptr or 0)
+        self._query_stream = None
 
     def set_triangles(self, tris: np.ndarray):
         tris = np.ascontiguousarray(tris, dtype=TRIANGLE)
@@ -477,6 +482,88 @@ class Backend:
         self._chk(self.L.rt_trace_rays(self.h, _ptr(o), _ptr(d), C.c_int64(n), _ptr(tri), _ptr(dst),
                                        _ptr(bu), _ptr(bv)))
         return tri, dst, bu, bv
+
+    # ---- ray queries on CUDA tensors (rt_query_closest / rt_query_occluded)
+    def _stream_for_queries(self, torch):
+        """The torch view of the stream the ctx launches on.  The ctx is bound once: to the stream given to
+        set_stream, or else to a private stream made here (rt_set_stream synchronises the previous stream, so it is
+        never called per query)."""
+        if self._query_stream is None:
+            dev = torch.device("cuda", self.cfg.device)
+            if self._stream_ptr:
+                self._query_stream = torch.cuda.ExternalStream(self._stream_ptr, device=dev)
+            else:
+                s = torch.cuda.Stream(device=dev)
+                self.set_stream(s.cuda_stream)
+                self._query_stream = s
+        return self._query_stream
+
+    def _query_inputs(self, torch, origins, dirs, tmax):
+        dev = torch.device("cuda", self.cfg.device)
+
+        def check(t, what, shape):
+            if not isinstance(t, torch.Tensor):
+                raise BackendError(f"{what} must be a torch tensor")
+            if t.device != dev:
+                raise BackendError(f"{what} is on {t.device}, the backend's device is {dev}")
+            if t.dtype != torch.float32:
+                raise BackendError(f"{what} must be float32, not {t.dtype}")
+            if tuple(t.shape) != shape:
+                raise BackendError(f"{what} has shape {tuple(t.shape)}, expected {shape}")
+            return t.contiguous()
+
+        n = origins.shape[0] if isinstance(origins, torch.Tensor) and origins.dim() == 2 else -1
+        if n < 0:
+            raise BackendError("origins must be a float32 (N, 3) CUDA tensor")
+        o = check(origins, "origins", (n, 3))
+        d = check(dirs, "dirs", (n, 3))
+        if tmax is None:
+            tm = None
+        elif isinstance(tmax, (int, float)) and not isinstance(tmax, bool):
+            tm = torch.full((n,), float(tmax), dtype=torch.float32, device=dev)
+        else:
+            tm = check(tmax, "tmax", (n,))
+        return n, o, d, tm
+
+    def _run_query(self, torch, fn, tensors, args):
+        """Enqueue one query ordered after the current torch stream's work and before whatever it does next, with no
+        host synchronisation: the query stream waits for the current stream, the current stream waits for the query."""
+        cur = torch.cuda.current_stream(torch.device("cuda", self.cfg.device))
+        qs = self._stream_for_queries(torch)
+        qs.wait_stream(cur)
+        self._chk(fn(self.h, *args))
+        cur.wait_stream(qs)
+        for t in tensors:   # the caching allocator must not hand these out again before the query has run
+            if t is not None:
+                t.record_stream(qs)
+
+    @staticmethod
+    def _dptr(t):
+        return C.c_void_p(None if t is None else t.data_ptr())
+
+    def query_closest(self, origins, dirs, tmax=None):
+        """Closest hit of every ray on the device: origins / dirs float32 (N, 3) CUDA tensors; tmax None (unbounded),
+        a float or a float32 (N,) tensor.  Returns (tri_id int32, dst, u, v), (N,) tensors: the result of trace_rays
+        for the same ray when its distance is below tmax, else the miss -1 / 1e38 / 0 / 0."""
+        import torch
+        n, o, d, tm = self._query_inputs(torch, origins, dirs, tmax)
+        dev = o.device
+        tri = torch.empty(n, dtype=torch.int32, device=dev)
+        dst, bu, bv = (torch.empty(n, dtype=torch.float32, device=dev) for _ in range(3))
+        self._run_query(torch, self.L.rt_query_closest, (o, d, tm, tri, dst, bu, bv),
+                        (self._dptr(o), self._dptr(d), self._dptr(tm), C.c_int64(n), self._dptr(tri),
+                         self._dptr(dst), self._dptr(bu), self._dptr(bv)))
+        return tri, dst, bu, bv
+
+    def query_occluded(self, origins, dirs, tmax=None):
+        """Is anything hit with t < tmax?  Same inputs as query_closest; returns a bool (N,) CUDA tensor.  The walk
+        stops at the first triangle it accepts."""
+        import torch
+        n, o, d, tm = self._query_inputs(torch, origins, dirs, tmax)
+        occ = torch.empty(n, dtype=torch.bool, device=o.device)   # one byte per element, written as 0 / 1
+        self._run_query(torch, self.L.rt_query_occluded, (o, d, tm, occ),
+                        (self._dptr(o), self._dptr(d), self._dptr(tm), C.c_int64(n), self._dptr(occ)))
+        return occ
 
     def get_bvh(self):
         nn, nt = C.c_int64(), C.c_int64()

@@ -8,6 +8,7 @@
 #include <cstdlib>
 #include <cmath>
 #include <cstring>
+#include <initializer_list>
 #include <new>
 #include <string>
 #include <vector>
@@ -110,6 +111,8 @@ struct rt_ctx {
     int sm_count = 148;
     int extend_blocks_per_sm = 4;
     int extend_blocks_per_sm_wide = 8;
+    int query_blocks_per_sm[2][2] = {{4, 8}, {4, 8}};  // k_extend's query variants: [ANY][4-wide]
+    DevBuf d_query;                // the queries' [0] ray count, [1] work cursor (allocated by rt_create)
     int use_ploc = 1, shade_blocks_per_sm = 64;
     int hooks_thread = 0;          // RT_HOOKS=thread: parity hooks walk the binary tree per thread (preview's code path)
     int bvh_width = 4;             // 4: k_extend walks 4-wide nodes collapsed from the binary tree; 2: the binary tree (RT_BVH_WIDTH)
@@ -226,6 +229,8 @@ Launcher make_launcher(rt_ctx* ctx, const rt_uniforms* u = nullptr) {
     L.instrument = ctx->cfg.instrument != 0;
     L.extend_grid = ctx->sm_count * ctx->extend_blocks_per_sm;
     L.extend_grid_wide = ctx->sm_count * ctx->extend_blocks_per_sm_wide;
+    for (int a = 0; a < 2; a++)
+        for (int w = 0; w < 2; w++) L.query_grid[a][w] = ctx->sm_count * ctx->query_blocks_per_sm[a][w];
     L.shade_blocks_per_sm = ctx->shade_blocks_per_sm;
     L.kernel_launches = &ctx->kernel_launches;
     L.extend_launches = &ctx->extend_launches;
@@ -576,6 +581,10 @@ int rt_create(rt_ctx** out, const rt_config* cfg) {
     ctx->stream = ctx->own_stream;
     ctx->extend_blocks_per_sm = wf_extend_blocks_per_sm(cfg->instrument != 0, false);
     ctx->extend_blocks_per_sm_wide = wf_extend_blocks_per_sm(cfg->instrument != 0, true);
+    for (int w = 0; w < 2; w++) {
+        ctx->query_blocks_per_sm[0][w] = wf_extend_blocks_per_sm(cfg->instrument != 0, w == 1, Query::CLOSEST);
+        ctx->query_blocks_per_sm[1][w] = wf_extend_blocks_per_sm(cfg->instrument != 0, w == 1, Query::ANY);
+    }
     {
         // Path slots: fewer, larger wavefronts amortise the drain of the persistent kernels (config 2: 8 lanes
         // per pixel 1203 ms/step, 64 lanes 1057 ms; round 2: 128 Mi slots 744.8 ms, 512 Mi — the whole 4-frame
@@ -593,7 +602,8 @@ int rt_create(rt_ctx** out, const rt_config* cfg) {
     if (const char* e5 = getenv("RT_BVH_BUILDER")) ctx->use_ploc = strcmp(e5, "lbvh") != 0;
     if (const char* e14 = getenv("RT_HOOKS")) ctx->hooks_thread = strcmp(e14, "thread") == 0;
     if (ctx->d_stats.reserve(4 * sizeof(unsigned long long)) != cudaSuccess ||
-        cudaMemsetAsync(ctx->d_stats.p, 0, 4 * sizeof(unsigned long long), ctx->stream) != cudaSuccess) {
+        cudaMemsetAsync(ctx->d_stats.p, 0, 4 * sizeof(unsigned long long), ctx->stream) != cudaSuccess ||
+        ctx->d_query.reserve(2 * sizeof(uint32_t)) != cudaSuccess) {
         delete ctx;
         return fail(nullptr, RT_ERR_CUDA, "rt_create: cannot allocate counters");
     }
@@ -948,6 +958,59 @@ int rt_trace_rays(rt_ctx* ctx, const float* origins, const float* dirs, int64_t 
     if (bu) CK(cudaMemcpyAsync(bu, ctx->d_scratch[4].p, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     if (bv) CK(cudaMemcpyAsync(bv, ctx->d_scratch[5].p, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
+    return RT_OK;
+}
+
+namespace {
+// Everything a ray query checks before it enqueues anything.  The arrays must be device (or managed) memory of the
+// ctx's device: k_extend reads and writes them in place.
+int validate_query(rt_ctx* ctx, const char* fn, const float* o, const float* d, const float* tmax, int64_t count,
+                   std::initializer_list<const void*> outputs) {
+    if (!ctx->built) return fail(ctx, RT_ERR_STATE, "scene not built: call rt_scene_build first");
+    if (count < 0) return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": count < 0");
+    if (count > ((int64_t)1 << 30)) return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": more than 2^30 rays in one call");
+    if (count == 0) return RT_OK;
+    if (!o || !d) return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": NULL origins or dirs");
+    auto on_device = [&](const void* p) {
+        cudaPointerAttributes a;
+        if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+            cudaGetLastError();
+            return false;
+        }
+        return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == ctx->cfg.device;
+    };
+    for (const void* p : {(const void*)o, (const void*)d, (const void*)tmax})
+        if (p && !on_device(p))
+            return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": an input is not device memory of device " +
+                                                 std::to_string(ctx->cfg.device));
+    for (const void* p : outputs)
+        if (p && !on_device(p))
+            return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": an output is not device memory of device " +
+                                                 std::to_string(ctx->cfg.device));
+    return RT_OK;
+}
+}  // namespace
+
+int rt_query_closest(rt_ctx* ctx, const float* origins, const float* dirs, const float* tmax, int64_t count,
+                     int32_t* tri_id, float* dst, float* bu, float* bv) {
+    GUARD();
+    int rc = validate_query(ctx, "rt_query_closest", origins, dirs, tmax, count, {tri_id, dst, bu, bv});
+    if (rc || count == 0) return rc;
+    const QueryArgs q{origins, dirs, tmax, tri_id, dst, bu, bv, nullptr};
+    CK(wf_query(make_launcher(ctx), make_view(ctx), q, count, Query::CLOSEST, ctx->d_query.as<uint32_t>(),
+                ctx->d_stats.as<unsigned long long>()));
+    return RT_OK;
+}
+
+int rt_query_occluded(rt_ctx* ctx, const float* origins, const float* dirs, const float* tmax, int64_t count,
+                      uint8_t* occluded) {
+    GUARD();
+    if (count > 0 && !occluded) return fail(ctx, RT_ERR_INVALID, "rt_query_occluded: NULL occluded");
+    int rc = validate_query(ctx, "rt_query_occluded", origins, dirs, tmax, count, {occluded});
+    if (rc || count == 0) return rc;
+    const QueryArgs q{origins, dirs, tmax, nullptr, nullptr, nullptr, nullptr, occluded};
+    CK(wf_query(make_launcher(ctx), make_view(ctx), q, count, Query::ANY, ctx->d_query.as<uint32_t>(),
+                ctx->d_stats.as<unsigned long long>()));
     return RT_OK;
 }
 

@@ -116,6 +116,22 @@ struct HookBuffers {
     unsigned long long* stats;  // the ctx counters (segments, node visits, triangle tests)
 };
 
+// What k_extend computes.  RENDER: closest hit of every queued path, (t, u, v, sorted slot) into the hit records.
+// CLOSEST / ANY (rt_query_closest / rt_query_occluded): the caller's (N, 3) origin and direction arrays are read and
+// its outputs written in place, with a per-ray tmax; ANY stops a ray at the first triangle it accepts.
+enum class Query : int { RENDER = 0, CLOSEST = 1, ANY = 2 };
+// device pointers of one ray query (all of them caller memory; NULL tmax = unbounded, NULL closest outputs = skipped)
+struct QueryArgs {
+    const float* o3;
+    const float* d3;
+    const float* tmax;
+    int32_t* tri;
+    float* dst;
+    float* bu;
+    float* bv;
+    uint8_t* occluded;
+};
+
 struct Launcher {
     cudaStream_t st;
     int sm_count;
@@ -123,6 +139,7 @@ struct Launcher {
     bool instrument;
     int extend_grid;   // persistent k_extend grid: SMs x resident blocks per SM
     int extend_grid_wide;  // the same for the 4-wide variant (more registers)
+    int query_grid[2][2];  // the same for the query variants: [ANY][4-wide]
     bool widen_primary;  // camera rays may start far outside the quantisation grid (rt_scene.cuh, slab1)
     bool hooks_thread; // parity hooks walk the binary tree per thread instead of running k_extend
     int shade_blocks_per_sm;  // grid-stride k_shade: blocks per SM
@@ -136,7 +153,7 @@ struct Launcher {
     bool timing;
 };
 
-int wf_extend_blocks_per_sm(bool instrument, bool wide);
+int wf_extend_blocks_per_sm(bool instrument, bool wide, Query q = Query::RENDER);
 cudaError_t wf_clear_accum(const Launcher& L, const WaveBuffers& wb, long long entries);
 cudaError_t wf_seed_pixels(const Launcher& L, const SceneView& sc, const WaveBuffers& wb, const FrameParams& fp);
 cudaError_t wf_render_batch(const Launcher& L, const SceneView& sc, const WaveBuffers& wb, const FrameParams& fp);
@@ -147,6 +164,9 @@ cudaError_t wf_first_hit(const Launcher& L, const SceneView& sc, const FramePara
                          int32_t* tri_id, float* dst);
 cudaError_t wf_trace_rays(const Launcher& L, const SceneView& sc, const float* o, const float* d, int64_t n,
                           const HookBuffers& hb, int32_t* tri, float* dst, float* bu, float* bv);
+// n > 0 rays of `q` through k_extend (CLOSEST or ANY); counts = [0] rays, [1] work cursor (device words of the ctx)
+cudaError_t wf_query(const Launcher& L, const SceneView& sc, const QueryArgs& q, int64_t n, Query mode,
+                     uint32_t* counts, unsigned long long* stats);
 cudaError_t wf_scatter_rows(const Launcher& L, const uint32_t* compact, uint32_t* full, const int32_t* rows,
                             int nrows, int width);
 cudaError_t wf_gather_rows(const Launcher& L, const uint32_t* full, uint32_t* compact, const int32_t* rows,

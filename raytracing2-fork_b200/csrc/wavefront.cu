@@ -384,12 +384,20 @@ __device__ __forceinline__ bool is_leaf_code(int32_t x) { return x < 0 && (uint3
 // is a stale bestT while a leaf is parked (a few more node visits).  How far a lane runs ahead of its parked leaf
 // depends on the other lanes of its warp, so the instrumented variants (COUNT) walk without it: their node-visit
 // and triangle-test counts are those of each ray's own sequential walk.
-template <bool COUNT, bool WIDE, bool WIDEN>
+//
+// Q = CLOSEST / ANY serve the ray queries: the refill reads the caller's (N, 3) arrays and an optional tmax, the pop
+// phase writes the caller's outputs, and everything they add sits behind `if constexpr`, so the RENDER instantiations
+// compile as before (`qa` is appended to the parameters and never read by them).  The hit rule of a query: a triangle
+// counts iff 1e-6 < dst < min(tmax, kMissT).  bestT starts at the largest float below that bound, which turns the
+// traversal's `dst <= bestT` into `dst < bound` (DESIGN.md, "Ray queries").
+template <bool COUNT, bool WIDE, bool WIDEN, Query Q>
 __global__ void __launch_bounds__(kExtBlock, kExtMinBlocks) k_extend(const __grid_constant__ SceneView sc, PathArrays cur,
                                                       float4* __restrict__ hit, const uint32_t* __restrict__ count,
                                                       uint32_t* __restrict__ cursor,
-                                                      unsigned long long* __restrict__ stats) {
+                                                      unsigned long long* __restrict__ stats,
+                                                      const __grid_constant__ QueryArgs qa) {
     constexpr bool SPEC = !COUNT;
+    constexpr bool ANY = Q == Query::ANY;
     constexpr int kNodeSteps = WIDE ? 2 : 4;  // node steps per vote (3 on the 4-wide tree, 3 / 6 on the binary one: slower)
     const uint32_t n = *count;
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&stats[0], (unsigned long long)n);
@@ -417,9 +425,25 @@ __global__ void __launch_bounds__(kExtBlock, kExtMinBlocks) k_extend(const __gri
     int sp = 0;
     uint32_t visits = 0, tests = 0;
 
+    // the result of ray `i` (a query writes the caller's arrays; a miss is -1 / kMissT / 0 / 0, or "not occluded")
+    auto write_result = [&](uint32_t i) {
+        if constexpr (Q == Query::RENDER) {
+            hit[i] = make_float4(r.bestT, bestU, bestV, __int_as_float(bestSlot));
+        } else if constexpr (ANY) {
+            qa.occluded[i] = bestSlot >= 0 ? 1 : 0;
+        } else {
+            const bool h = bestSlot >= 0;
+            if (qa.tri) qa.tri[i] = h ? __ldg(&sc.tri_orig[bestSlot]) : -1;
+            if (qa.dst) qa.dst[i] = h ? r.bestT : kMissT;
+            if (qa.bu) qa.bu[i] = h ? bestU : 0.0f;
+            if (qa.bv) qa.bv[i] = h ? bestV : 0.0f;
+        }
+    };
     if (sc.num_tris <= 0) {  // empty scene: every ray misses
-        for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
-            hit[i] = make_float4(kMissT, 0.0f, 0.0f, __int_as_float(-1));
+        for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+            if constexpr (Q == Query::RENDER) hit[i] = make_float4(kMissT, 0.0f, 0.0f, __int_as_float(-1));
+            else write_result(i);
+        }
     }
 
     // exact Möller–Trumbore against every triangle of one leaf; min (dst, original index) wins
@@ -433,7 +457,15 @@ __global__ void __launch_bounds__(kExtBlock, kExtMinBlocks) k_extend(const __gri
             // candidate (the dependent 4-byte gather was 3.4 % of k_extend's stall samples)
             if (dst <= r.bestT && dst < kMissT) {
                 bool take = dst < r.bestT;
-                if (!take) take = __ldg(&sc.tri_orig[s]) < __ldg(&sc.tri_orig[bestSlot]);  // bestT < kMissT: bestSlot >= 0
+                if constexpr (Q == Query::RENDER) {
+                    if (!take) take = __ldg(&sc.tri_orig[s]) < __ldg(&sc.tri_orig[bestSlot]);  // bestT < kMissT: bestSlot >= 0
+                } else if constexpr (ANY) {
+                    take = true;  // any accepted triangle answers the query
+                } else {
+                    // a query's bestT starts at the bound itself (dst == bestT is a hit), so the first candidate
+                    // must be taken without the tie-break: there is no bestSlot to compare with yet
+                    if (!take) take = bestSlot < 0 || __ldg(&sc.tri_orig[s]) < __ldg(&sc.tri_orig[bestSlot]);
+                }
                 if (take) {
                     r.bestT = dst; bestU = u; bestV = v; bestSlot = s;
                 }
@@ -444,7 +476,19 @@ __global__ void __launch_bounds__(kExtBlock, kExtMinBlocks) k_extend(const __gri
         const int32_t packed = ~code;
         const int32_t first = packed & kLeafFirstMask;
         const int32_t cnt = (packed >> kLeafCountShift) + 1;
-        for (int32_t s = first; s < first + cnt; s++) test_tri(s);
+        for (int32_t s = first; s < first + cnt; s++) {
+            if constexpr (ANY) {
+                if (bestSlot >= 0) break;  // answered: the rest of the leaf (and a second leaf) is not tested
+            }
+            test_tri(s);
+        }
+    };
+    // ANY: a ray that accepted a triangle is done.  Its stack and parked leaf are dropped, and the pop phase writes
+    // the result and hands the lane to the refill.
+    auto any_done = [&]() {
+        if constexpr (ANY) {
+            if (bestSlot >= 0) { sp = 0; post = kNoLeaf; node = kPop; }
+        }
     };
     // (Round 2 measured the two leaves of a lane as ONE merged triangle sequence — the warp iterates max(cntA + cntB)
     // instead of max(cntA) + max(cntB): 5781 vs 5853 Mrays/s, the per-iteration select costs more than the shorter loop
@@ -497,7 +541,7 @@ __global__ void __launch_bounds__(kExtBlock, kExtMinBlocks) k_extend(const __gri
                 if (SPEC && post != kNoLeaf) {
                     node = kDrain;
                 } else {
-                    hit[ray] = make_float4(r.bestT, bestU, bestV, __int_as_float(bestSlot));
+                    write_result(ray);
                     node = kIdle;
                 }
             } else {  // (leaving this pop to the node iterations' select-based one: -1.9 %, the vote below needs it)
@@ -533,16 +577,32 @@ __global__ void __launch_bounds__(kExtBlock, kExtMinBlocks) k_extend(const __gri
                     have = i < fend;
                 }
                 if (have) {
-                    const float4 a = cur.od0[i];
-                    const float4 b = cur.od1[i];
                     ray = i;
-                    r.o = v3(a.x, a.y, a.z);
-                    r.d = v3(a.w, b.x, b.y);
+                    bool live = true;
+                    if constexpr (Q == Query::RENDER) {
+                        const float4 a = cur.od0[i];
+                        const float4 b = cur.od1[i];
+                        r.o = v3(a.x, a.y, a.z);
+                        r.d = v3(a.w, b.x, b.y);
+                        r.bestT = kMissT;
+                    } else {
+                        // 12-byte records: 32 consecutive rays of a warp read 384 contiguous bytes per array
+                        const size_t k = 3 * (size_t)i;
+                        r.o = v3(qa.o3[k], qa.o3[k + 1], qa.o3[k + 2]);
+                        r.d = v3(qa.d3[k], qa.d3[k + 1], qa.d3[k + 2]);
+                        const float tm = qa.tmax ? qa.tmax[i] : kMissT;
+                        // NaN, zero or negative tmax: no hit possible, the ray is not traversed.  (fminf in slab1
+                        // would ignore a NaN bound, so it must not reach bestT.)
+                        live = tm > 0.0f;
+                        const float bound = fminf(tm, kMissT);
+                        r.bestT = __int_as_float(__float_as_int(bound) - 1);  // largest float below the bound
+                    }
                     r.g = make_grid_ray(sc, r.o, r.d);
-                    r.bestT = kMissT; bestU = 0.0f; bestV = 0.0f; bestSlot = -1;
+                    bestU = 0.0f; bestV = 0.0f; bestSlot = -1;
                     sp = 0;
                     post = kNoLeaf;
                     node = sc.root_is_leaf ? pack_leaf(0, sc.num_tris) : 0;
+                    if (!live) node = kPop;
                     postpone();
                 }
             }
@@ -555,9 +615,10 @@ __global__ void __launch_bounds__(kExtBlock, kExtMinBlocks) k_extend(const __gri
                 nnext = next + min(want, avail);
                 nend = end;
             }
-            if (lane < 10u) {
+            if (Q == Query::RENDER && lane < 10u) {
                 // the records this warp takes at its NEXT refill are known exactly: the head of its private range
-                // (five 128-byte lines of each array cover 32 records wherever the range starts)
+                // (five 128-byte lines of each array cover 32 records wherever the range starts).  The queries do
+                // not prefetch.
                 const uint32_t p = nnext + 8u * (lane < 5u ? lane : lane - 5u);
                 const void* q = lane < 5u ? (const void*)&cur.od0[p] : (const void*)&cur.od1[p];
                 if (p < nend) prefetch_l2(q);
@@ -583,10 +644,12 @@ __global__ void __launch_bounds__(kExtBlock, kExtMinBlocks) k_extend(const __gri
                     if (is_leaf_code(node)) test_leaf(node);
                     post = kNoLeaf;
                     if (parked) node = kPop;
+                    any_done();
                 }
             } else if (parked) {
                 test_leaf(node);
                 node = kPop;
+                any_done();
             }
         } else {
             // several node steps per vote amortise the voting overhead.  When no lane can reach the end of the
@@ -1291,16 +1354,24 @@ struct Timed {
     }
 };
 
-int wf_extend_blocks_per_sm(bool instrument, bool wide) {
+template <Query Q>
+static int extend_blocks_per_sm(bool instrument, bool wide) {
+    // queries always widen (origins anywhere); rendering asks about its unwidened variant, as before
+    constexpr bool WD = Q != Query::RENDER;
     int nb = 0;
     cudaError_t e;
     if (wide)
-        e = instrument ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<true, true, true>, kExtBlock, 0)
-                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, true, false>, kExtBlock, 0);
+        e = instrument ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<true, true, true, Q>, kExtBlock, 0)
+                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, true, WD, Q>, kExtBlock, 0);
     else
-        e = instrument ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<true, false, true>, kExtBlock, 0)
-                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, false, false>, kExtBlock, 0);
+        e = instrument ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<true, false, true, Q>, kExtBlock, 0)
+                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, false, WD, Q>, kExtBlock, 0);
     return e == cudaSuccess && nb > 0 ? nb : 4;
+}
+int wf_extend_blocks_per_sm(bool instrument, bool wide, Query q) {
+    if (q == Query::CLOSEST) return extend_blocks_per_sm<Query::CLOSEST>(instrument, wide);
+    if (q == Query::ANY) return extend_blocks_per_sm<Query::ANY>(instrument, wide);
+    return extend_blocks_per_sm<Query::RENDER>(instrument, wide);
 }
 
 // One closest-hit pass over the `*count` rays of `rays` (od0 / od1): the persistent traversal kernel in the variant
@@ -1310,7 +1381,8 @@ static void launch_extend(const Launcher& L, const SceneView& sc, const PathArra
     const bool wide = sc.nodes4 != nullptr;
     const int grid = wide ? L.extend_grid_wide : L.extend_grid;
     cudaStream_t st = L.st;
-#define RT_EXT(C, W, WD) k_extend<C, W, WD><<<grid, kExtBlock, 0, st>>>(sc, rays, hit, count, cursor, stats)
+#define RT_EXT(C, W, WD) \
+    k_extend<C, W, WD, Query::RENDER><<<grid, kExtBlock, 0, st>>>(sc, rays, hit, count, cursor, stats, QueryArgs{})
     if (wide) {
         if (L.instrument) RT_EXT(true, true, true);
         else if (widen) RT_EXT(false, true, true);
@@ -1451,6 +1523,29 @@ cudaError_t wf_trace_rays(const Launcher& L, const SceneView& sc, const float* o
     launch_extend(L, sc, hb.rays, hb.hit, hb.counts, hb.counts + 1, true, hb.stats);
     k_unpack_hits<<<nblocks(n), kBlock, 0, L.st>>>(sc, hb.hit, n, tri, dst, bu, bv);
     (*L.kernel_launches) += 3;
+    return cudaGetLastError();
+}
+
+// The ray queries run k_extend straight on the caller's arrays: one tiny kernel resets the ctx's count and cursor
+// words on the stream, then the persistent traversal.  No staging, no copy, no host synchronisation.
+cudaError_t wf_query(const Launcher& L, const SceneView& sc, const QueryArgs& q, int64_t n, Query mode,
+                     uint32_t* counts, unsigned long long* stats) {
+    if (n <= 0) return cudaSuccess;
+    const bool wide = sc.nodes4 != nullptr, any = mode == Query::ANY;
+    const int grid = L.query_grid[any ? 1 : 0][wide ? 1 : 0];
+    k_hook_count<<<1, 32, 0, L.st>>>(counts, (uint32_t)n);
+    const PathArrays none{nullptr, nullptr, nullptr};
+#define RT_Q(C, W, QQ) k_extend<C, W, true, QQ><<<grid, kExtBlock, 0, L.st>>>(sc, none, nullptr, counts, counts + 1, stats, q)
+    if (any) {
+        if (wide) { if (L.instrument) RT_Q(true, true, Query::ANY); else RT_Q(false, true, Query::ANY); }
+        else { if (L.instrument) RT_Q(true, false, Query::ANY); else RT_Q(false, false, Query::ANY); }
+    } else {
+        if (wide) { if (L.instrument) RT_Q(true, true, Query::CLOSEST); else RT_Q(false, true, Query::CLOSEST); }
+        else { if (L.instrument) RT_Q(true, false, Query::CLOSEST); else RT_Q(false, false, Query::CLOSEST); }
+    }
+#undef RT_Q
+    (*L.kernel_launches) += 2;
+    (*L.extend_launches)++;
     return cudaGetLastError();
 }
 
