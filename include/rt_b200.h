@@ -282,6 +282,22 @@ int rt_query_closest(rt_ctx* ctx, const float* origins, const float* dirs, const
 int rt_query_occluded(rt_ctx* ctx, const float* origins, const float* dirs, const float* tmax, int64_t count,
                       uint8_t* occluded);
 
+/* ---------------------------------------------------------------- nearest-triangle queries on device memory
+ * For each point p (points: count*3 floats) and radius r = max_dist[i] (max_dist: count floats, or NULL = unbounded):
+ * among the triangles T with dist(p, T) < min(r, 1e38), the one with the smallest distance to the CLOSED triangle
+ * (interior, edges, vertices; a distance of 0 is a hit); exact ties go to the lowest id.  Outputs per point: tri_id
+ * (index into the array given to rt_scene_set_triangles), dist, bary_u / bary_v with closest point a + (b-a) u +
+ * (c-a) v, and that point (closest: count*3 floats).  A miss writes -1 / 1e38 / 0 / 0 and (0, 0, 0).  A NaN, zero
+ * or negative radius and a point with a non-finite coordinate never hit.  A distance whose square overflows binary32
+ * (beyond about 1.8e19) is +inf and never hits.  The point-triangle distance is defined, bit for bit, by the CPU
+ * oracle (DESIGN.md §5).  Sorting the points for spatial coherence is left to the caller.
+ * Same rules as the ray queries: asynchronous on the ctx stream, every non-NULL pointer must be device (or managed)
+ * memory of cfg.device and points must not be NULL, else RT_ERR_INVALID, as are count < 0 and count > 2^30, all
+ * rejected before anything is enqueued; count == 0 returns RT_OK and launches nothing; an unbuilt scene returns
+ * RT_ERR_STATE.  Outputs may be NULL (not written). */
+int rt_query_nearest(rt_ctx* ctx, const float* points, const float* max_dist, int64_t count, int32_t* tri_id,
+                     float* dist, float* bary_u, float* bary_v, float* closest);
+
 /* Export the GPU-built BVH: call with nodes == NULL to get sizes.  sorted_tri_ids[slot] = original
  * triangle index stored at that leaf slot. */
 int rt_scene_get_bvh(rt_ctx* ctx, rt_bvh_node* nodes, int64_t* node_count, int32_t* sorted_tri_ids,

@@ -174,7 +174,7 @@ ABI_SYMBOLS = [
     "rt_scene_set_triangles", "rt_scene_set_materials", "rt_scene_set_texture", "rt_scene_build",
     "rt_render_frame", "rt_read_frame_rgba32f", "rt_screenshot", "rt_screenshot_device",
     "rt_screenshot_fetch", "rt_screenshot_partial", "rt_read_frame_sum", "rt_finalize_sums", "rt_first_hit", "rt_trace_rays",
-    "rt_query_closest", "rt_query_occluded", "rt_scene_get_bvh", "rt_get_counters",
+    "rt_query_closest", "rt_query_occluded", "rt_query_nearest", "rt_scene_get_bvh", "rt_get_counters",
     "rt_reset_counters", "rt_comm_unique_id", "rt_comm_init", "rt_split_rows", "rt_split_frames", "rt_plan_batches",
 ]
 
@@ -483,7 +483,7 @@ class Backend:
                                        _ptr(bu), _ptr(bv)))
         return tri, dst, bu, bv
 
-    # ---- ray queries on CUDA tensors (rt_query_closest / rt_query_occluded)
+    # ---- queries on CUDA tensors (rt_query_closest / rt_query_occluded / rt_query_nearest)
     def _stream_for_queries(self, torch):
         """The torch view of the stream the ctx launches on.  The ctx is bound once: to the stream given to
         set_stream, or else to a private stream made here (rt_set_stream synchronises the previous stream, so it is
@@ -498,7 +498,9 @@ class Backend:
                 self._query_stream = s
         return self._query_stream
 
-    def _query_inputs(self, torch, origins, dirs, tmax):
+    def _query_inputs(self, torch, inputs, bound, bound_name):
+        """inputs: (name, tensor) pairs, each a float32 (N, 3) CUDA tensor, the first defining N; bound (tmax or
+        max_dist): None, a float or a float32 (N,) CUDA tensor.  Returns N, the contiguous inputs and the bound."""
         dev = torch.device("cuda", self.cfg.device)
 
         def check(t, what, shape):
@@ -512,18 +514,18 @@ class Backend:
                 raise BackendError(f"{what} has shape {tuple(t.shape)}, expected {shape}")
             return t.contiguous()
 
-        n = origins.shape[0] if isinstance(origins, torch.Tensor) and origins.dim() == 2 else -1
+        first_name, first = inputs[0]
+        n = first.shape[0] if isinstance(first, torch.Tensor) and first.dim() == 2 else -1
         if n < 0:
-            raise BackendError("origins must be a float32 (N, 3) CUDA tensor")
-        o = check(origins, "origins", (n, 3))
-        d = check(dirs, "dirs", (n, 3))
-        if tmax is None:
-            tm = None
-        elif isinstance(tmax, (int, float)) and not isinstance(tmax, bool):
-            tm = torch.full((n,), float(tmax), dtype=torch.float32, device=dev)
+            raise BackendError(f"{first_name} must be a float32 (N, 3) CUDA tensor")
+        arrays = [check(t, name, (n, 3)) for name, t in inputs]
+        if bound is None:
+            b = None
+        elif isinstance(bound, (int, float)) and not isinstance(bound, bool):
+            b = torch.full((n,), float(bound), dtype=torch.float32, device=dev)
         else:
-            tm = check(tmax, "tmax", (n,))
-        return n, o, d, tm
+            b = check(bound, bound_name, (n,))
+        return n, arrays, b
 
     def _run_query(self, torch, fn, tensors, args):
         """Enqueue one query ordered after the current torch stream's work and before whatever it does next, with no
@@ -546,7 +548,7 @@ class Backend:
         a float or a float32 (N,) tensor.  Returns (tri_id int32, dst, u, v), (N,) tensors: the result of trace_rays
         for the same ray when its distance is below tmax, else the miss -1 / 1e38 / 0 / 0."""
         import torch
-        n, o, d, tm = self._query_inputs(torch, origins, dirs, tmax)
+        n, (o, d), tm = self._query_inputs(torch, (("origins", origins), ("dirs", dirs)), tmax, "tmax")
         dev = o.device
         tri = torch.empty(n, dtype=torch.int32, device=dev)
         dst, bu, bv = (torch.empty(n, dtype=torch.float32, device=dev) for _ in range(3))
@@ -559,11 +561,28 @@ class Backend:
         """Is anything hit with t < tmax?  Same inputs as query_closest; returns a bool (N,) CUDA tensor.  The walk
         stops at the first triangle it accepts."""
         import torch
-        n, o, d, tm = self._query_inputs(torch, origins, dirs, tmax)
+        n, (o, d), tm = self._query_inputs(torch, (("origins", origins), ("dirs", dirs)), tmax, "tmax")
         occ = torch.empty(n, dtype=torch.bool, device=o.device)   # one byte per element, written as 0 / 1
         self._run_query(torch, self.L.rt_query_occluded, (o, d, tm, occ),
                         (self._dptr(o), self._dptr(d), self._dptr(tm), C.c_int64(n), self._dptr(occ)))
         return occ
+
+    def query_nearest(self, points, max_dist=None):
+        """Nearest triangle of every point on the device: points a float32 (N, 3) CUDA tensor; max_dist None
+        (unbounded), a float or a float32 (N,) tensor.  Returns (tri_id int32, dist, u, v, closest (N, 3)): among the
+        triangles closer than max_dist (and 1e38), the nearest one, exact ties to the lowest id, with the barycentrics
+        of the closest point a + (b - a) u + (c - a) v and that point; a miss is -1 / 1e38 / 0 / 0 / (0, 0, 0).  A NaN,
+        zero or negative max_dist and a non-finite point miss.  Ordered on the current stream like query_closest."""
+        import torch
+        n, (p,), md = self._query_inputs(torch, (("points", points),), max_dist, "max_dist")
+        dev = p.device
+        tri = torch.empty(n, dtype=torch.int32, device=dev)
+        dist, bu, bv = (torch.empty(n, dtype=torch.float32, device=dev) for _ in range(3))
+        closest = torch.empty((n, 3), dtype=torch.float32, device=dev)
+        self._run_query(torch, self.L.rt_query_nearest, (p, md, tri, dist, bu, bv, closest),
+                        (self._dptr(p), self._dptr(md), C.c_int64(n), self._dptr(tri), self._dptr(dist),
+                         self._dptr(bu), self._dptr(bv), self._dptr(closest)))
+        return tri, dist, bu, bv, closest
 
     def get_bvh(self):
         nn, nt = C.c_int64(), C.c_int64()

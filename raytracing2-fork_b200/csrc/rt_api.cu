@@ -962,15 +962,17 @@ int rt_trace_rays(rt_ctx* ctx, const float* origins, const float* dirs, int64_t 
 }
 
 namespace {
-// Everything a ray query checks before it enqueues anything.  The arrays must be device (or managed) memory of the
-// ctx's device: k_extend reads and writes them in place.
-int validate_query(rt_ctx* ctx, const char* fn, const float* o, const float* d, const float* tmax, int64_t count,
-                   std::initializer_list<const void*> outputs) {
+// Everything a query checks before it enqueues anything.  `inputs` (named `what`) must not be NULL, `bound` (tmax or
+// max_dist) may be.  The arrays must be device (or managed) memory of the ctx's device: the kernels read and write
+// them in place.
+int validate_query(rt_ctx* ctx, const char* fn, const char* what, std::initializer_list<const float*> inputs,
+                   const float* bound, int64_t count, std::initializer_list<const void*> outputs) {
     if (!ctx->built) return fail(ctx, RT_ERR_STATE, "scene not built: call rt_scene_build first");
     if (count < 0) return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": count < 0");
-    if (count > ((int64_t)1 << 30)) return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": more than 2^30 rays in one call");
+    if (count > ((int64_t)1 << 30)) return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": more than 2^30 queries in one call");
     if (count == 0) return RT_OK;
-    if (!o || !d) return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": NULL origins or dirs");
+    for (const float* p : inputs)
+        if (!p) return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": NULL " + what);
     auto on_device = [&](const void* p) {
         cudaPointerAttributes a;
         if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
@@ -979,10 +981,11 @@ int validate_query(rt_ctx* ctx, const char* fn, const float* o, const float* d, 
         }
         return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == ctx->cfg.device;
     };
-    for (const void* p : {(const void*)o, (const void*)d, (const void*)tmax})
-        if (p && !on_device(p))
-            return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": an input is not device memory of device " +
-                                                 std::to_string(ctx->cfg.device));
+    bool inputs_ok = !bound || on_device(bound);
+    for (const float* p : inputs) inputs_ok = inputs_ok && on_device(p);
+    if (!inputs_ok)
+        return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": an input is not device memory of device " +
+                                             std::to_string(ctx->cfg.device));
     for (const void* p : outputs)
         if (p && !on_device(p))
             return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": an output is not device memory of device " +
@@ -994,7 +997,7 @@ int validate_query(rt_ctx* ctx, const char* fn, const float* o, const float* d, 
 int rt_query_closest(rt_ctx* ctx, const float* origins, const float* dirs, const float* tmax, int64_t count,
                      int32_t* tri_id, float* dst, float* bu, float* bv) {
     GUARD();
-    int rc = validate_query(ctx, "rt_query_closest", origins, dirs, tmax, count, {tri_id, dst, bu, bv});
+    int rc = validate_query(ctx, "rt_query_closest", "origins or dirs", {origins, dirs}, tmax, count, {tri_id, dst, bu, bv});
     if (rc || count == 0) return rc;
     const QueryArgs q{origins, dirs, tmax, tri_id, dst, bu, bv, nullptr};
     CK(wf_query(make_launcher(ctx), make_view(ctx), q, count, Query::CLOSEST, ctx->d_query.as<uint32_t>(),
@@ -1006,11 +1009,21 @@ int rt_query_occluded(rt_ctx* ctx, const float* origins, const float* dirs, cons
                       uint8_t* occluded) {
     GUARD();
     if (count > 0 && !occluded) return fail(ctx, RT_ERR_INVALID, "rt_query_occluded: NULL occluded");
-    int rc = validate_query(ctx, "rt_query_occluded", origins, dirs, tmax, count, {occluded});
+    int rc = validate_query(ctx, "rt_query_occluded", "origins or dirs", {origins, dirs}, tmax, count, {occluded});
     if (rc || count == 0) return rc;
     const QueryArgs q{origins, dirs, tmax, nullptr, nullptr, nullptr, nullptr, occluded};
     CK(wf_query(make_launcher(ctx), make_view(ctx), q, count, Query::ANY, ctx->d_query.as<uint32_t>(),
                 ctx->d_stats.as<unsigned long long>()));
+    return RT_OK;
+}
+
+int rt_query_nearest(rt_ctx* ctx, const float* points, const float* max_dist, int64_t count, int32_t* tri_id,
+                     float* dist, float* bu, float* bv, float* closest) {
+    GUARD();
+    int rc = validate_query(ctx, "rt_query_nearest", "points", {points}, max_dist, count, {tri_id, dist, bu, bv, closest});
+    if (rc || count == 0) return rc;
+    const NearestArgs q{points, max_dist, tri_id, dist, bu, bv, closest};
+    CK(wf_nearest(make_launcher(ctx), make_view(ctx), q, count, ctx->d_stats.as<unsigned long long>()));
     return RT_OK;
 }
 

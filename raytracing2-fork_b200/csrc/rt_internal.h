@@ -132,6 +132,18 @@ struct QueryArgs {
     uint8_t* occluded;
 };
 
+// device pointers of one nearest-triangle query (rt_query_nearest; all caller memory, NULL max_dist = unbounded, NULL
+// outputs = skipped)
+struct NearestArgs {
+    const float* points;    // count * 3
+    const float* max_dist;  // count
+    int32_t* tri;
+    float* dist;
+    float* bu;
+    float* bv;
+    float* closest;         // count * 3
+};
+
 struct Launcher {
     cudaStream_t st;
     int sm_count;
@@ -171,5 +183,10 @@ cudaError_t wf_scatter_rows(const Launcher& L, const uint32_t* compact, uint32_t
                             int nrows, int width);
 cudaError_t wf_gather_rows(const Launcher& L, const uint32_t* full, uint32_t* compact, const int32_t* rows,
                            int nrows, int width);
+
+// ---------------------------------------------------------------- nearest.cu
+// n > 0 points through k_nearest, one thread per point, on L.st
+cudaError_t wf_nearest(const Launcher& L, const SceneView& sc, const NearestArgs& q, int64_t n,
+                       unsigned long long* stats);
 
 }  // namespace rt
