@@ -251,7 +251,9 @@ int rt_read_frame_sum(rt_ctx* ctx, uint32_t* sums_bottom_up);
 int rt_finalize_sums(rt_ctx* ctx, const uint32_t* sums_bottom_up, int32_t width, int32_t height,
                      int32_t frames, uint8_t* rgb8_topdown);
 
-/* ---------------------------------------------------------------- parity hooks */
+/* ---------------------------------------------------------------- parity hooks
+ * Host-memory entry points that return when their results are in the caller's arrays.  Both are the closest-hit
+ * query (rt_query_closest with no tmax) run on device copies of the rays, so they report exactly what it reports. */
 /* Closest hit of the primary ray of every pixel: tri_id[y*W+x] = index into the array given to
  * rt_scene_set_triangles, or -1 for a miss; dst = hit distance (1e38f for a miss).  Row 0 = bottom.
  * Ties in dst are broken by the lowest triangle index. */

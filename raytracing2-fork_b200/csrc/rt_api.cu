@@ -114,7 +114,6 @@ struct rt_ctx {
     int query_blocks_per_sm[2][2] = {{4, 8}, {4, 8}};  // k_extend's query variants: [ANY][4-wide]
     DevBuf d_query;                // the queries' [0] ray count, [1] work cursor (allocated by rt_create)
     int use_ploc = 1, shade_blocks_per_sm = 64;
-    int hooks_thread = 0;          // RT_HOOKS=thread: parity hooks walk the binary tree per thread (preview's code path)
     int bvh_width = 4;             // 4: k_extend walks 4-wide nodes collapsed from the binary tree; 2: the binary tree (RT_BVH_WIDTH)
     DevBuf d_wide_count;           // [0] wide nodes written, [1] worst-case traversal stack entries (k_collapse4)
     uint32_t wide_nodes = 0;
@@ -156,7 +155,7 @@ struct rt_ctx {
     // wavefront
     DevBuf d_path[6], d_hit, d_contrib, d_accum, d_pixrng, d_counts, d_stats, d_image, d_sum, d_out, d_rows;
     DevBuf d_stage, d_compact;  // tile-split gather
-    DevBuf d_scratch[10];       // first-hit / trace-rays staging: in, out, ray queue, hits, counts
+    DevBuf d_scratch[6];        // staging of host arrays (parity hooks: origins, directions, tri_id, dst, u, v)
     int width = 0, height = 0;
     std::vector<int32_t> rows;  // rows this rank owns (tile split)
     int last_frames = 0;
@@ -222,7 +221,6 @@ Launcher make_launcher(rt_ctx* ctx, const rt_uniforms* u = nullptr) {
     Launcher L;
     L.st = ctx->stream;
     L.widen_primary = u ? widen_needed(ctx, *u) : true;
-    L.hooks_thread = ctx->hooks_thread != 0;
 
     L.sm_count = ctx->sm_count;
     L.rng_mode = ctx->cfg.rng_mode;
@@ -600,7 +598,6 @@ int rt_create(rt_ctx** out, const rt_config* cfg) {
     if (const char* e8 = getenv("RT_MAX_PATHS_MI")) ctx->default_budget = (uint64_t)std::max(1, atoi(e8)) << 20;
     if (const char* e9 = getenv("RT_BVH_WIDTH")) ctx->bvh_width = atoi(e9) == 4 ? 4 : 2;
     if (const char* e5 = getenv("RT_BVH_BUILDER")) ctx->use_ploc = strcmp(e5, "lbvh") != 0;
-    if (const char* e14 = getenv("RT_HOOKS")) ctx->hooks_thread = strcmp(e14, "thread") == 0;
     if (ctx->d_stats.reserve(4 * sizeof(unsigned long long)) != cudaSuccess ||
         cudaMemsetAsync(ctx->d_stats.p, 0, 4 * sizeof(unsigned long long), ctx->stream) != cudaSuccess ||
         ctx->d_query.reserve(2 * sizeof(uint32_t)) != cudaSuccess) {
@@ -733,7 +730,7 @@ int rt_scene_build(rt_ctx* ctx) {
     CK(ctx->d_grid.reserve(6 * sizeof(float)));
     CK(ctx->d_wide_count.reserve(2 * sizeof(uint32_t)));
     {
-        // one arena, in the order the traversal touches it: binary nodes (hooks, preview, RT_BVH_WIDTH=2) | 4-wide
+        // one arena, in the order the traversal touches it: binary nodes (preview, RT_BVH_WIDTH=2) | 4-wide
         // nodes | triangle records | original indices | shading records.  The L2 persisting window covers what
         // k_extend gathers from: [wide nodes (or binary nodes when there are none), end of the original indices).
         auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
@@ -893,16 +890,14 @@ int rt_screenshot(rt_ctx* ctx, const rt_uniforms* uniforms, int32_t frames, uint
 }
 
 namespace {
-// queue, hit records and counters for a hook over n rays (d_scratch[6..9])
-int hook_buffers(rt_ctx* ctx, size_t n, HookBuffers* hb) {
-    CK(ctx->d_scratch[6].reserve(n * sizeof(float4)));
-    CK(ctx->d_scratch[7].reserve(n * sizeof(float4)));
-    CK(ctx->d_scratch[8].reserve(n * sizeof(float4)));
-    CK(ctx->d_scratch[9].reserve(2 * sizeof(uint32_t)));
-    hb->rays = PathArrays{ctx->d_scratch[6].as<float4>(), ctx->d_scratch[7].as<float4>(), nullptr};
-    hb->hit = ctx->d_scratch[8].as<float4>();
-    hb->counts = ctx->d_scratch[9].as<uint32_t>();
-    hb->stats = ctx->d_stats.as<unsigned long long>();
+// Closest hit of n rays whose (N, 3) origins and directions are in device memory: k_extend's CLOSEST query, on the ctx
+// stream, with the ctx's count and cursor words.  rt_query_closest passes the caller's arrays, the parity hooks
+// their staged copies and no tmax.
+int closest_query(rt_ctx* ctx, const float* o3, const float* d3, const float* tmax, int64_t n, int32_t* tri,
+                  float* dst, float* bu, float* bv) {
+    const QueryArgs q{o3, d3, tmax, tri, dst, bu, bv, nullptr};
+    CK(wf_query(make_launcher(ctx), make_view(ctx), q, n, Query::CLOSEST, ctx->d_query.as<uint32_t>(),
+                ctx->d_stats.as<unsigned long long>()));
     return RT_OK;
 }
 }  // namespace
@@ -913,21 +908,21 @@ int rt_first_hit(rt_ctx* ctx, const rt_uniforms* uniforms, int32_t mode, int32_t
     if (rc) return rc;
     if (mode != RT_FIRST_HIT_CENTRE && mode != RT_FIRST_HIT_SAMPLE0) return fail(ctx, RT_ERR_INVALID, "rt_first_hit: bad mode");
     const size_t n = (size_t)uniforms->width * uniforms->height;
-    CK(ctx->d_scratch[0].reserve(n * sizeof(int32_t)));
-    CK(ctx->d_scratch[1].reserve(n * sizeof(float)));
-    HookBuffers hb;
-    rc = hook_buffers(ctx, n, &hb);
-    if (rc) return rc;
-    Launcher L = make_launcher(ctx);
-    SceneView sc = make_view(ctx);
+    CK(ctx->d_scratch[0].reserve(n * 3 * sizeof(float)));
+    CK(ctx->d_scratch[1].reserve(n * 3 * sizeof(float)));
+    CK(ctx->d_scratch[2].reserve(n * sizeof(int32_t)));
+    CK(ctx->d_scratch[3].reserve(n * sizeof(float)));
     FrameParams fp;
     memset(&fp, 0, sizeof fp);
     fp.u = *uniforms;
     fp.width = (int)uniforms->width;
     fp.height = (int)uniforms->height;
-    CK(wf_first_hit(L, sc, fp, mode, hb, ctx->d_scratch[0].as<int32_t>(), ctx->d_scratch[1].as<float>()));
-    if (tri_id) CK(cudaMemcpyAsync(tri_id, ctx->d_scratch[0].p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    if (dst) CK(cudaMemcpyAsync(dst, ctx->d_scratch[1].p, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(wf_first_rays(make_launcher(ctx), fp, mode, ctx->d_scratch[0].as<float>(), ctx->d_scratch[1].as<float>()));
+    rc = closest_query(ctx, ctx->d_scratch[0].as<float>(), ctx->d_scratch[1].as<float>(), nullptr, (int64_t)n,
+                       ctx->d_scratch[2].as<int32_t>(), ctx->d_scratch[3].as<float>(), nullptr, nullptr);
+    if (rc) return rc;
+    if (tri_id) CK(cudaMemcpyAsync(tri_id, ctx->d_scratch[2].p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    if (dst) CK(cudaMemcpyAsync(dst, ctx->d_scratch[3].p, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return RT_OK;
 }
@@ -943,16 +938,12 @@ int rt_trace_rays(rt_ctx* ctx, const float* origins, const float* dirs, int64_t 
     CK(ctx->d_scratch[0].reserve(n * 3 * sizeof(float)));
     CK(ctx->d_scratch[1].reserve(n * 3 * sizeof(float)));
     for (int i = 2; i < 6; i++) CK(ctx->d_scratch[i].reserve(n * sizeof(float)));
-    HookBuffers hb;
-    int rc = hook_buffers(ctx, n, &hb);
-    if (rc) return rc;
     CK(cudaMemcpyAsync(ctx->d_scratch[0].p, origins, n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemcpyAsync(ctx->d_scratch[1].p, dirs, n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-    Launcher L = make_launcher(ctx);
-    SceneView sc = make_view(ctx);
-    CK(wf_trace_rays(L, sc, ctx->d_scratch[0].as<float>(), ctx->d_scratch[1].as<float>(), count, hb,
-                     ctx->d_scratch[2].as<int32_t>(), ctx->d_scratch[3].as<float>(), ctx->d_scratch[4].as<float>(),
-                     ctx->d_scratch[5].as<float>()));
+    const int rc = closest_query(ctx, ctx->d_scratch[0].as<float>(), ctx->d_scratch[1].as<float>(), nullptr, count,
+                                 ctx->d_scratch[2].as<int32_t>(), ctx->d_scratch[3].as<float>(),
+                                 ctx->d_scratch[4].as<float>(), ctx->d_scratch[5].as<float>());
+    if (rc) return rc;
     if (tri_id) CK(cudaMemcpyAsync(tri_id, ctx->d_scratch[2].p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
     if (dst) CK(cudaMemcpyAsync(dst, ctx->d_scratch[3].p, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     if (bu) CK(cudaMemcpyAsync(bu, ctx->d_scratch[4].p, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
@@ -999,10 +990,7 @@ int rt_query_closest(rt_ctx* ctx, const float* origins, const float* dirs, const
     GUARD();
     int rc = validate_query(ctx, "rt_query_closest", "origins or dirs", {origins, dirs}, tmax, count, {tri_id, dst, bu, bv});
     if (rc || count == 0) return rc;
-    const QueryArgs q{origins, dirs, tmax, tri_id, dst, bu, bv, nullptr};
-    CK(wf_query(make_launcher(ctx), make_view(ctx), q, count, Query::CLOSEST, ctx->d_query.as<uint32_t>(),
-                ctx->d_stats.as<unsigned long long>()));
-    return RT_OK;
+    return closest_query(ctx, origins, dirs, tmax, count, tri_id, dst, bu, bv);
 }
 
 int rt_query_occluded(rt_ctx* ctx, const float* origins, const float* dirs, const float* tmax, int64_t count,

@@ -108,19 +108,13 @@ struct WaveBuffers {
     uint8_t* out_rgb8;    // W*H*3 final, top-down
 };
 
-// queue + results of the parity hooks (rt_first_hit, rt_trace_rays), which run k_extend on caller-defined rays
-struct HookBuffers {
-    PathArrays rays;            // od0 / od1 only
-    float4* hit;
-    uint32_t* counts;           // [0] rays, [1] work cursor
-    unsigned long long* stats;  // the ctx counters (segments, node visits, triangle tests)
-};
-
 // What k_extend computes.  RENDER: closest hit of every queued path, (t, u, v, sorted slot) into the hit records.
 // CLOSEST / ANY (rt_query_closest / rt_query_occluded): the caller's (N, 3) origin and direction arrays are read and
-// its outputs written in place, with a per-ray tmax; ANY stops a ray at the first triangle it accepts.
+// its outputs written in place, with a per-ray tmax; ANY stops a ray at the first triangle it accepts.  The parity
+// hooks (rt_first_hit, rt_trace_rays) are CLOSEST with no tmax on device copies staged by rt_api.cu.
 enum class Query : int { RENDER = 0, CLOSEST = 1, ANY = 2 };
-// device pointers of one ray query (all of them caller memory; NULL tmax = unbounded, NULL closest outputs = skipped)
+// device pointers of one ray query (caller memory, or the hooks' staging; NULL tmax = unbounded, NULL closest outputs =
+// skipped)
 struct QueryArgs {
     const float* o3;
     const float* d3;
@@ -153,7 +147,6 @@ struct Launcher {
     int extend_grid_wide;  // the same for the 4-wide variant (more registers)
     int query_grid[2][2];  // the same for the query variants: [ANY][4-wide]
     bool widen_primary;  // camera rays may start far outside the quantisation grid (rt_scene.cuh, slab1)
-    bool hooks_thread; // parity hooks walk the binary tree per thread instead of running k_extend
     int shade_blocks_per_sm;  // grid-stride k_shade: blocks per SM
     uint64_t* kernel_launches;
     uint64_t* extend_launches;
@@ -172,10 +165,8 @@ cudaError_t wf_render_batch(const Launcher& L, const SceneView& sc, const WaveBu
 cudaError_t wf_resolve_frame(const Launcher& L, const WaveBuffers& wb, const FrameParams& fp, bool add_to_sum);
 cudaError_t wf_preview(const Launcher& L, const SceneView& sc, const WaveBuffers& wb, const FrameParams& fp);
 cudaError_t wf_finalize(const Launcher& L, const uint32_t* frame_sum, uint8_t* out, int w, int h, int frames);
-cudaError_t wf_first_hit(const Launcher& L, const SceneView& sc, const FrameParams& fp, int mode, const HookBuffers& hb,
-                         int32_t* tri_id, float* dst);
-cudaError_t wf_trace_rays(const Launcher& L, const SceneView& sc, const float* o, const float* d, int64_t n,
-                          const HookBuffers& hb, int32_t* tri, float* dst, float* bu, float* bv);
+// rt_first_hit's width x height camera rays as (N, 3) origin and direction arrays (device)
+cudaError_t wf_first_rays(const Launcher& L, const FrameParams& fp, int mode, float* o3, float* d3);
 // n > 0 rays of `q` through k_extend (CLOSEST or ANY); counts = [0] rays, [1] work cursor (device words of the ctx)
 cudaError_t wf_query(const Launcher& L, const SceneView& sc, const QueryArgs& q, int64_t n, Query mode,
                      uint32_t* counts, unsigned long long* stats);

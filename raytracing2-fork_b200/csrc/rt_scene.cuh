@@ -16,7 +16,7 @@
 //              144 B, compute.glsl:425,443-444.)
 //   nodes4   : 64 B per 4-wide node (two 256-bit loads), collapsed from the binary tree by k_collapse4: four child
 //              boxes w0..w11 (three words each, same quantisation), four children w12..w15.  k_extend walks these by
-//              default; the binary nodes serve the per-thread hooks, RT_BVH_WIDTH=2 and the deep-tree fallback.
+//              default; the binary nodes serve the preview kernel, RT_BVH_WIDTH=2 and the deep-tree fallback.
 //   tri_geom : 64 B stride per sorted triangle; traversal reads the first 48 B = a, e0 = b-a,
 //              e1 = c-a, N = cross(e0,e1), precomputed with the very operations
 //              compute.glsl:307-309 performs per test, so every bit of dst,u,v is unchanged
@@ -204,9 +204,7 @@ __host__ __device__ __forceinline__ int32_t pack_leaf(int32_t first, int32_t cou
 // a subtree is skipped when its (conservatively widened) slab interval cannot contain a hit with
 // t <= best, so the result equals the exhaustive minimum over all triangles regardless of the
 // hierarchy or the visiting order.
-template <bool COUNT>
-__device__ __forceinline__ HitRec closest_hit(const SceneView& sc, V3 o, V3 d, uint32_t& nodeVisits,
-                                              uint32_t& triTests) {
+__device__ __forceinline__ HitRec closest_hit(const SceneView& sc, V3 o, V3 d) {
     HitRec best;
     best.t = kMissT;
     best.u = 0.0f;
@@ -227,7 +225,6 @@ __device__ __forceinline__ HitRec closest_hit(const SceneView& sc, V3 o, V3 d, u
         if (cur >= 0) {
             uint32_t w[8];
             ldg256u(sc.nodes + 2 * cur, w);
-            if (COUNT) nodeVisits++;
             float lNear, rNear;
             bool hitL, hitR;
             slab2(w, g, best.t, lNear, rNear, hitL, hitR);
@@ -252,7 +249,6 @@ __device__ __forceinline__ HitRec closest_hit(const SceneView& sc, V3 o, V3 d, u
             const int32_t count = (packed >> kLeafCountShift) + 1;
             for (int32_t s = first; s < first + count; s++) {
                 const TriGeom tg = load_tri(sc, s);
-                if (COUNT) triTests++;
                 float dst, u, v;
                 if (ray_triangle(o, d, tg.a, tg.e0, tg.e1, tg.N, dst, u, v)) {
                     if (dst <= best.t && dst < kMissT) {

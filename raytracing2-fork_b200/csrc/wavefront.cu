@@ -12,7 +12,7 @@
 //   k_resolve       S:696-700   mean, ACES, gamma, image store; + unorm8 quantise and add (R:194-238)
 //   k_finalize      R:248-259   average of the 8-bit frames, truncate, flip
 //   k_preview       S:565-645   traceBasic, one thread per pixel (interactive preview)
-//   k_first_hit / k_trace_rays  parity hooks
+//   k_first_rays                the camera rays of the first-hit parity hook, traced by k_extend's CLOSEST query
 //
 // A "path slot" is (lane, pixel): a batch holds frames_in_batch x samples_in_batch lanes of every pixel
 // (FrameParams, rt_internal.h) and each slot owns one float4 of `contrib`; the radiance of a path is a single value written at its
@@ -1148,12 +1148,12 @@ __global__ void __launch_bounds__(kBlock) k_preview(const __grid_constant__ Scen
     bool insideGlass = false;
     V3 cum = v3(0.0f, 0.0f, 0.0f);
     int bounceCount = 0;
-    uint32_t nv = 0, nt = 0, segs = 0;
+    uint32_t segs = 0;
     V3 result = v3(0.0f, 0.0f, 0.0f);
     bool done = false;
     while (bounceCount < fp.u.maxBounceCount && !done) {
         bounceCount++;
-        const HitRec h = closest_hit<false>(sc, o, d, nv, nt);
+        const HitRec h = closest_hit(sc, o, d);
         segs++;
         if (h.slot >= 0) {
             const V3 hitPoint = o + d * h.t;
@@ -1180,7 +1180,7 @@ __global__ void __launch_bounds__(kBlock) k_preview(const __grid_constant__ Scen
                     cum = cum + color;
                     if (fp.u.basicShadingShadow != 0) {
                         const V3 toLight = normalize(v3(fp.u.basicShadingLightPosition) - hitPoint);
-                        const HitRec sh = closest_hit<false>(sc, o, toLight, nv, nt);
+                        const HitRec sh = closest_hit(sc, o, toLight);
                         segs++;
                         const V3 c = sh.slot >= 0 ? cum / 5.0f : cum;
                         result = c / (float)bounceCount;
@@ -1221,12 +1221,11 @@ __global__ void __launch_bounds__(kBlock) k_preview(const __grid_constant__ Scen
     if ((threadIdx.x & 31) == 0) atomicAdd(&stats[0], (unsigned long long)segs);
 }
 
-// ---- parity hooks.  Since round 2 they run the TIMED traversal kernel: the rays are packed into a queue, k_extend
-// finds the closest hits, and a small kernel turns (t, u, v, sorted slot) into what the C-ABI reports.  (With
-// RT_HOOKS=thread they use the per-thread binary-tree walk `closest_hit` of rt_scene.cuh instead, the code path of
-// the preview kernel — the two must agree, tests/test_gpu_parity.py.)
+// ---- parity hooks.  rt_first_hit and rt_trace_rays are the closest-hit query (wf_query, Query::CLOSEST) on staged
+// copies; this kernel writes rt_first_hit's camera rays as the (N, 3) origin and direction arrays the query reads.
 template <int MODE>
-__global__ void __launch_bounds__(kBlock) k_first_rays(const __grid_constant__ FrameParams fp, int mode, PathArrays rays) {
+__global__ void __launch_bounds__(kBlock) k_first_rays(const __grid_constant__ FrameParams fp, int mode,
+                                                       float* __restrict__ o3, float* __restrict__ d3) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= fp.width * fp.height) return;
     const int ty = p / fp.width, tx = p - ty * fp.width;
@@ -1241,85 +1240,18 @@ __global__ void __launch_bounds__(kBlock) k_first_rays(const __grid_constant__ F
         rng.stream(0u);
         sample_ray(fp.u, ps, rng, o, d);
     }
-    rays.od0[p] = make_float4(o.x, o.y, o.z, d.x);
-    rays.od1[p] = make_float4(d.y, d.z, 0.0f, 0.0f);
-}
-__global__ void __launch_bounds__(kBlock) k_pack_rays(const float* __restrict__ o3, const float* __restrict__ d3,
-                                                      long long n, PathArrays rays) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    rays.od0[i] = make_float4(o3[3 * i], o3[3 * i + 1], o3[3 * i + 2], d3[3 * i]);
-    rays.od1[i] = make_float4(d3[3 * i + 1], d3[3 * i + 2], 0.0f, 0.0f);
-}
-__global__ void __launch_bounds__(kBlock) k_unpack_hits(const __grid_constant__ SceneView sc,
-                                                        const float4* __restrict__ hit, long long n,
-                                                        int32_t* __restrict__ tri, float* __restrict__ dst,
-                                                        float* __restrict__ bu, float* __restrict__ bv) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const float4 h = hit[i];
-    const int32_t slot = __float_as_int(h.w);
-    if (tri) tri[i] = slot >= 0 ? __ldg(&sc.tri_orig[slot]) : -1;
-    if (dst) dst[i] = h.x;
-    if (bu) bu[i] = slot >= 0 ? h.y : 0.0f;
-    if (bv) bv[i] = slot >= 0 ? h.z : 0.0f;
+    const size_t k = 3 * (size_t)p;  // 64-bit: 3 * p wraps in 32 bits above 715 827 882 pixels
+    o3[k] = o.x;
+    o3[k + 1] = o.y;
+    o3[k + 2] = o.z;
+    d3[k] = d.x;
+    d3[k + 1] = d.y;
+    d3[k + 2] = d.z;
 }
 __global__ void k_hook_count(uint32_t* counts, uint32_t n) {
     if (threadIdx.x == 0) {
         counts[0] = n;   // rays in the queue
         counts[1] = 0u;  // k_extend's work cursor
-    }
-}
-
-template <int MODE>
-__global__ void __launch_bounds__(kBlock) k_first_hit(const __grid_constant__ SceneView sc,
-                                                      const __grid_constant__ FrameParams fp, int mode,
-                                                      int32_t* __restrict__ tri_id, float* __restrict__ dst) {
-    const int p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= fp.width * fp.height) return;
-    const int ty = p / fp.width, tx = p - ty * fp.width;
-    const PixelSetup ps = pixel_setup(fp.u, tx, ty);
-    V3 o, d;
-    if (mode == RT_FIRST_HIT_CENTRE) {
-        o = v3(fp.u.cameraPos);
-        d = ps.centreDir;
-    } else {
-        Rng<MODE> rng;
-        rng.init(MODE == 0 ? ps.seed : 0u, ps.pixelId, fp.u.frameIndex, 0u);
-        rng.stream(0u);
-        sample_ray(fp.u, ps, rng, o, d);
-    }
-    uint32_t nv = 0, nt = 0;
-    const HitRec h = closest_hit<false>(sc, o, d, nv, nt);
-    tri_id[p] = h.slot >= 0 ? __ldg(&sc.tri_orig[h.slot]) : -1;
-    dst[p] = h.t;
-}
-
-template <bool COUNT>
-__global__ void __launch_bounds__(kBlock) k_trace_rays(const __grid_constant__ SceneView sc,
-                                                       const float* __restrict__ o3, const float* __restrict__ d3,
-                                                       long long n, int32_t* __restrict__ tri, float* __restrict__ dst,
-                                                       float* __restrict__ bu, float* __restrict__ bv,
-                                                       unsigned long long* __restrict__ stats) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    uint32_t nv = 0, nt = 0;
-    if (i < n) {
-        const HitRec h = closest_hit<COUNT>(sc, v3(o3 + 3 * i), v3(d3 + 3 * i), nv, nt);
-        if (tri) tri[i] = h.slot >= 0 ? __ldg(&sc.tri_orig[h.slot]) : -1;
-        if (dst) dst[i] = h.t;
-        if (bu) bu[i] = h.slot >= 0 ? h.u : 0.0f;
-        if (bv) bv[i] = h.slot >= 0 ? h.v : 0.0f;
-    }
-    if (COUNT) {
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            nv += __shfl_xor_sync(0xffffffffu, nv, off);
-            nt += __shfl_xor_sync(0xffffffffu, nt, off);
-        }
-        if ((threadIdx.x & 31) == 0) {
-            atomicAdd(&stats[2], (unsigned long long)nv);
-            atomicAdd(&stats[3], (unsigned long long)nt);
-        }
     }
 }
 
@@ -1485,48 +1417,17 @@ cudaError_t wf_finalize(const Launcher& L, const uint32_t* frame_sum, uint8_t* o
     return cudaGetLastError();
 }
 
-cudaError_t wf_first_hit(const Launcher& L, const SceneView& sc, const FrameParams& fp, int mode, const HookBuffers& hb,
-                         int32_t* tri_id, float* dst) {
+cudaError_t wf_first_rays(const Launcher& L, const FrameParams& fp, int mode, float* o3, float* d3) {
     const long long n = (long long)fp.width * fp.height;
-    if (L.hooks_thread) {
-        if (L.rng_mode == RT_RNG_REF_PCG)
-            k_first_hit<0><<<nblocks(n), kBlock, 0, L.st>>>(sc, fp, mode, tri_id, dst);
-        else
-            k_first_hit<1><<<nblocks(n), kBlock, 0, L.st>>>(sc, fp, mode, tri_id, dst);
-        (*L.kernel_launches)++;
-        return cudaGetLastError();
-    }
     if (L.rng_mode == RT_RNG_REF_PCG)
-        k_first_rays<0><<<nblocks(n), kBlock, 0, L.st>>>(fp, mode, hb.rays);
+        k_first_rays<0><<<nblocks(n), kBlock, 0, L.st>>>(fp, mode, o3, d3);
     else
-        k_first_rays<1><<<nblocks(n), kBlock, 0, L.st>>>(fp, mode, hb.rays);
-    k_hook_count<<<1, 32, 0, L.st>>>(hb.counts, (uint32_t)n);
-    launch_extend(L, sc, hb.rays, hb.hit, hb.counts, hb.counts + 1, true, hb.stats);
-    k_unpack_hits<<<nblocks(n), kBlock, 0, L.st>>>(sc, hb.hit, n, tri_id, dst, nullptr, nullptr);
-    (*L.kernel_launches) += 3;
+        k_first_rays<1><<<nblocks(n), kBlock, 0, L.st>>>(fp, mode, o3, d3);
+    (*L.kernel_launches)++;
     return cudaGetLastError();
 }
 
-cudaError_t wf_trace_rays(const Launcher& L, const SceneView& sc, const float* o, const float* d, int64_t n,
-                          const HookBuffers& hb, int32_t* tri, float* dst, float* bu, float* bv) {
-    if (n <= 0) return cudaSuccess;
-    if (L.hooks_thread) {
-        if (L.instrument)
-            k_trace_rays<true><<<nblocks(n), kBlock, 0, L.st>>>(sc, o, d, n, tri, dst, bu, bv, hb.stats);
-        else
-            k_trace_rays<false><<<nblocks(n), kBlock, 0, L.st>>>(sc, o, d, n, tri, dst, bu, bv, hb.stats);
-        (*L.kernel_launches)++;
-        return cudaGetLastError();
-    }
-    k_pack_rays<<<nblocks(n), kBlock, 0, L.st>>>(o, d, n, hb.rays);
-    k_hook_count<<<1, 32, 0, L.st>>>(hb.counts, (uint32_t)n);
-    launch_extend(L, sc, hb.rays, hb.hit, hb.counts, hb.counts + 1, true, hb.stats);
-    k_unpack_hits<<<nblocks(n), kBlock, 0, L.st>>>(sc, hb.hit, n, tri, dst, bu, bv);
-    (*L.kernel_launches) += 3;
-    return cudaGetLastError();
-}
-
-// The ray queries run k_extend straight on the caller's arrays: one tiny kernel resets the ctx's count and cursor
+// The ray queries run k_extend straight on the arrays they are given: one tiny kernel resets the ctx's count and cursor
 // words on the stream, then the persistent traversal.  No staging, no copy, no host synchronisation.
 cudaError_t wf_query(const Launcher& L, const SceneView& sc, const QueryArgs& q, int64_t n, Query mode,
                      uint32_t* counts, unsigned long long* stats) {

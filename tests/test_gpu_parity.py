@@ -656,14 +656,15 @@ def test_real_asset_robot_if_generated():
 
 
 # ------------------------------------------------------------------------------------------------ round 2
-@pytest.mark.parametrize("env", [{"RT_HOOKS": "thread"}, {"RT_BVH_WIDTH": "2"}, {"RT_MAX_PATHS_MI": "1"},
+@pytest.mark.parametrize("env", [{"RT_BVH_WIDTH": "2"}, {"RT_MAX_PATHS_MI": "1"},
                                  {"RT_BVH_BUILDER": "lbvh"}, {"RT_BVH_BUILDER": "lbvh", "RT_BVH_WIDTH": "2"}])
 @pytest.mark.parametrize("rng_mode", [rt.RNG_REF_PCG, rt.RNG_PHILOX])
 def test_kernel_variants_change_no_bit(monkeypatch, env, rng_mode):
-    """The per-thread hooks, the binary tree, the Karras builder and a tiny path budget only reorder or re-route work:
-    frame, first-hit map and random rays must equal the oracle bit for bit under every switch (the defaults are covered
-    by every other test).  Both append policies of k_shade run in every case: the material zoo has no textures, so every
-    bounce defers its queue append; the textured mirror scene defers bounce 0 and appends the later bounces at once."""
+    """The binary tree, the Karras builder and a tiny path budget only reorder or re-route work: frame, first-hit map,
+    random rays and the shadowed preview frame (the per-thread walk over the binary tree) must equal the oracle bit for
+    bit under every switch (the defaults are covered by every other test).  Both append policies of k_shade run in every
+    case: the material zoo has no textures, so every bounce defers its queue append; the textured mirror scene defers
+    bounce 0 and appends the later bounces at once."""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     zoo = scenes.material_zoo()
@@ -683,6 +684,10 @@ def test_kernel_variants_change_no_bit(monkeypatch, env, rng_mode):
         b = orc.trace_rays(o, d, use_bvh=False)
         assert np.array_equal(a[0], b[0]) and np.array_equal(bits(a[1]), bits(b[1]))
         assert np.array_equal(bits(a[2]), bits(b[2])) and np.array_equal(bits(a[3]), bits(b[3]))
+        up = rt.interactive_uniforms(scene, cam)
+        up["basicShadingShadow"] = 1
+        be.render_frame(up)
+        assert_image_equal(be.read_frame(), orc.render_frame(up), f"preview, variant {env}")
         be.close()
 
 
