@@ -109,9 +109,7 @@ constexpr int kMaxBounces = 4096;
 struct rt_ctx {
     rt_config cfg{};
     int sm_count = 148;
-    int extend_blocks_per_sm = 4;
-    int extend_blocks_per_sm_wide = 8;
-    int query_blocks_per_sm[2][2] = {{4, 8}, {4, 8}};  // k_extend's query variants: [ANY][4-wide]
+    ExtendResidency extend_residency{};
     DevBuf d_query;                // the queries' [0] ray count, [1] work cursor (allocated by rt_create)
     int use_ploc = 1, shade_blocks_per_sm = 64;
     int bvh_width = 4;             // 4: k_extend walks 4-wide nodes collapsed from the binary tree; 2: the binary tree (RT_BVH_WIDTH)
@@ -225,10 +223,7 @@ Launcher make_launcher(rt_ctx* ctx, const rt_uniforms* u = nullptr) {
     L.sm_count = ctx->sm_count;
     L.rng_mode = ctx->cfg.rng_mode;
     L.instrument = ctx->cfg.instrument != 0;
-    L.extend_grid = ctx->sm_count * ctx->extend_blocks_per_sm;
-    L.extend_grid_wide = ctx->sm_count * ctx->extend_blocks_per_sm_wide;
-    for (int a = 0; a < 2; a++)
-        for (int w = 0; w < 2; w++) L.query_grid[a][w] = ctx->sm_count * ctx->query_blocks_per_sm[a][w];
+    L.extend_residency = &ctx->extend_residency;
     L.shade_blocks_per_sm = ctx->shade_blocks_per_sm;
     L.kernel_launches = &ctx->kernel_launches;
     L.extend_launches = &ctx->extend_launches;
@@ -570,6 +565,12 @@ int rt_create(rt_ctx** out, const rt_config* cfg) {
     cudaSetDevice(cfg->device);
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, cfg->device) == cudaSuccess) ctx->sm_count = prop.multiProcessorCount;
+    // fails only when the library has no image this device can load, which every launch would report too
+    e = wf_extend_residency(cfg->instrument != 0, &ctx->extend_residency);
+    if (e != cudaSuccess) {
+        delete ctx;
+        return fail(nullptr, RT_ERR_CUDA, std::string("rt_create: k_extend occupancy: ") + cudaGetErrorString(e));
+    }
     e = cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
         std::string m = std::string("rt_create: cudaStreamCreate: ") + cudaGetErrorString(e);
@@ -577,12 +578,6 @@ int rt_create(rt_ctx** out, const rt_config* cfg) {
         return fail(nullptr, RT_ERR_CUDA, m);
     }
     ctx->stream = ctx->own_stream;
-    ctx->extend_blocks_per_sm = wf_extend_blocks_per_sm(cfg->instrument != 0, false);
-    ctx->extend_blocks_per_sm_wide = wf_extend_blocks_per_sm(cfg->instrument != 0, true);
-    for (int w = 0; w < 2; w++) {
-        ctx->query_blocks_per_sm[0][w] = wf_extend_blocks_per_sm(cfg->instrument != 0, w == 1, Query::CLOSEST);
-        ctx->query_blocks_per_sm[1][w] = wf_extend_blocks_per_sm(cfg->instrument != 0, w == 1, Query::ANY);
-    }
     {
         // Path slots: fewer, larger wavefronts amortise the drain of the persistent kernels (config 2: 8 lanes
         // per pixel 1203 ms/step, 64 lanes 1057 ms; round 2: 128 Mi slots 744.8 ms, 512 Mi — the whole 4-frame
@@ -1092,7 +1087,8 @@ int rt_get_counters(rt_ctx* ctx, rt_counters* out) {
     out->bvh_bytes = out->bvh_nodes * 32 + (uint64_t)ctx->n_tris * 48;
     out->bvh_depth = ctx->bvh_depth;
     out->bvh_width = 2;
-    out->extend_blocks_per_sm = (uint64_t)ctx->extend_blocks_per_sm;
+    // rendering's k_extend after bounce 0: the counted walk when instrumented, else the one without widening
+    out->extend_blocks_per_sm = (uint64_t)ctx->extend_residency.blocks_per_sm[(int)Query::RENDER][ctx->wide_ok][0];
     out->bvh_stack_need = ctx->bvh_depth;
     out->bvh_build_rounds = ctx->build_rounds;
     if (ctx->wide_ok) {  // what k_extend walks: the 4-wide tree
@@ -1100,7 +1096,6 @@ int rt_get_counters(rt_ctx* ctx, rt_counters* out) {
         out->bvh_bytes = (uint64_t)ctx->wide_nodes * 64 + (uint64_t)ctx->n_tris * 48;
         out->bvh_depth = (uint64_t)ctx->wide_depth;
         out->bvh_width = 4;
-        out->extend_blocks_per_sm = (uint64_t)ctx->extend_blocks_per_sm_wide;
         out->bvh_stack_need = ctx->wide_stack_need;
     }
     return RT_OK;

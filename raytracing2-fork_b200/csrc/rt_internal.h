@@ -138,14 +138,18 @@ struct NearestArgs {
     float* closest;         // count * 3
 };
 
+// Resident 128-thread blocks per SM of the k_extend instantiation a launch picks, indexed [Q][4-wide][widen] like that
+// choice (wavefront.cu, extend_kernel).  Filled once per ctx; a persistent k_extend grid is SMs x this.
+struct ExtendResidency {
+    int blocks_per_sm[3][2][2];
+};
+
 struct Launcher {
     cudaStream_t st;
     int sm_count;
     int rng_mode;
     bool instrument;
-    int extend_grid;   // persistent k_extend grid: SMs x resident blocks per SM
-    int extend_grid_wide;  // the same for the 4-wide variant (more registers)
-    int query_grid[2][2];  // the same for the query variants: [ANY][4-wide]
+    const ExtendResidency* extend_residency;  // of the variants `instrument` selects
     bool widen_primary;  // camera rays may start far outside the quantisation grid (rt_scene.cuh, slab1)
     int shade_blocks_per_sm;  // grid-stride k_shade: blocks per SM
     uint64_t* kernel_launches;
@@ -158,7 +162,8 @@ struct Launcher {
     bool timing;
 };
 
-int wf_extend_blocks_per_sm(bool instrument, bool wide, Query q = Query::RENDER);
+// fills `r` from the occupancy of each k_extend instantiation a ctx with this `instrument` setting launches
+cudaError_t wf_extend_residency(bool instrument, ExtendResidency* r);
 cudaError_t wf_clear_accum(const Launcher& L, const WaveBuffers& wb, long long entries);
 cudaError_t wf_seed_pixels(const Launcher& L, const SceneView& sc, const WaveBuffers& wb, const FrameParams& fp);
 cudaError_t wf_render_batch(const Launcher& L, const SceneView& sc, const WaveBuffers& wb, const FrameParams& fp);

@@ -1248,7 +1248,8 @@ __global__ void __launch_bounds__(kBlock) k_first_rays(const __grid_constant__ F
     d3[k + 1] = d.y;
     d3[k + 2] = d.z;
 }
-__global__ void k_hook_count(uint32_t* counts, uint32_t n) {
+// ---- ray queries (wf_query): the ctx's count and cursor words, reset on the stream before each query
+__global__ void k_query_reset(uint32_t* counts, uint32_t n) {
     if (threadIdx.x == 0) {
         counts[0] = n;   // rays in the queue
         counts[1] = 0u;  // k_extend's work cursor
@@ -1286,45 +1287,43 @@ struct Timed {
     }
 };
 
-template <Query Q>
-static int extend_blocks_per_sm(bool instrument, bool wide) {
-    // queries always widen (origins anywhere); rendering asks about its unwidened variant, as before
-    constexpr bool WD = Q != Query::RENDER;
-    int nb = 0;
-    cudaError_t e;
-    if (wide)
-        e = instrument ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<true, true, true, Q>, kExtBlock, 0)
-                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, true, WD, Q>, kExtBlock, 0);
-    else
-        e = instrument ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<true, false, true, Q>, kExtBlock, 0)
-                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_extend<false, false, WD, Q>, kExtBlock, 0);
-    return e == cudaSuccess && nb > 0 ? nb : 4;
+using ExtendKernel = void (*)(SceneView, PathArrays, float4*, const uint32_t*, uint32_t*, unsigned long long*, QueryArgs);
+template <bool COUNT, bool WIDE>
+static ExtendKernel widened_extend(Query q) {
+    if (q == Query::CLOSEST) return k_extend<COUNT, WIDE, true, Query::CLOSEST>;
+    if (q == Query::ANY) return k_extend<COUNT, WIDE, true, Query::ANY>;
+    return k_extend<COUNT, WIDE, true, Query::RENDER>;
 }
-int wf_extend_blocks_per_sm(bool instrument, bool wide, Query q) {
-    if (q == Query::CLOSEST) return extend_blocks_per_sm<Query::CLOSEST>(instrument, wide);
-    if (q == Query::ANY) return extend_blocks_per_sm<Query::ANY>(instrument, wide);
-    return extend_blocks_per_sm<Query::RENDER>(instrument, wide);
+// The k_extend instantiation for one launch.  `wide`: the scene has the 4-wide tree.  `widen`: origins may lie far
+// outside the quantisation grid (rt_scene.cuh, slab1).
+static ExtendKernel extend_kernel(bool instrument, bool wide, bool widen, Query q) {
+    // the counted walk and the queries always take the widened slab test: only uninstrumented rendering has a variant
+    // without it
+    widen |= instrument || q != Query::RENDER;
+    if (!widen) return wide ? k_extend<false, true, false, Query::RENDER> : k_extend<false, false, false, Query::RENDER>;
+    if (instrument) return wide ? widened_extend<true, true>(q) : widened_extend<true, false>(q);
+    return wide ? widened_extend<false, true>(q) : widened_extend<false, false>(q);
 }
 
-// One closest-hit pass over the `*count` rays of `rays` (od0 / od1): the persistent traversal kernel in the variant
-// the scene and the launch call for.  `widen`: origins may lie far outside the quantisation grid (rt_scene.cuh).
-static void launch_extend(const Launcher& L, const SceneView& sc, const PathArrays& rays, float4* hit,
-                          const uint32_t* count, uint32_t* cursor, bool widen, unsigned long long* stats) {
+cudaError_t wf_extend_residency(bool instrument, ExtendResidency* r) {
+    for (int q = 0; q < 3; q++)
+        for (int w = 0; w < 2; w++)
+            for (int wd = 0; wd < 2; wd++) {
+                const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(
+                    &r->blocks_per_sm[q][w][wd], extend_kernel(instrument, w, wd, (Query)q), kExtBlock, 0);
+                if (e != cudaSuccess) return e;
+            }
+    return cudaSuccess;
+}
+
+// One persistent pass of k_extend over the `*count` rays: the instantiation extend_kernel picks, on a grid sized from
+// that instantiation's residency.  RENDER reads `rays` (od0 / od1) and writes `hit`; the queries read and write `qa`.
+static void launch_extend(const Launcher& L, const SceneView& sc, bool widen, Query q, const PathArrays& rays,
+                          float4* hit, const uint32_t* count, uint32_t* cursor, unsigned long long* stats,
+                          const QueryArgs& qa) {
     const bool wide = sc.nodes4 != nullptr;
-    const int grid = wide ? L.extend_grid_wide : L.extend_grid;
-    cudaStream_t st = L.st;
-#define RT_EXT(C, W, WD) \
-    k_extend<C, W, WD, Query::RENDER><<<grid, kExtBlock, 0, st>>>(sc, rays, hit, count, cursor, stats, QueryArgs{})
-    if (wide) {
-        if (L.instrument) RT_EXT(true, true, true);
-        else if (widen) RT_EXT(false, true, true);
-        else RT_EXT(false, true, false);
-    } else {
-        if (L.instrument) RT_EXT(true, false, true);
-        else if (widen) RT_EXT(false, false, true);
-        else RT_EXT(false, false, false);
-    }
-#undef RT_EXT
+    const int grid = L.sm_count * L.extend_residency->blocks_per_sm[(int)q][wide][widen];
+    extend_kernel(L.instrument, wide, widen, q)<<<grid, kExtBlock, 0, L.st>>>(sc, rays, hit, count, cursor, stats, qa);
     (*L.kernel_launches)++;
     (*L.extend_launches)++;
 }
@@ -1362,7 +1361,8 @@ cudaError_t wf_render_batch(const Launcher& L, const SceneView& sc, const WaveBu
         {
             Timed t(L, 0);
             // camera rays may start far outside the scene; every later segment starts on a surface of it
-            launch_extend(L, sc, a, wb.hit, wb.counts + bounce, cursors + bounce, bounce == 0 && L.widen_primary, wb.stats);
+            launch_extend(L, sc, bounce == 0 && L.widen_primary, Query::RENDER, a, wb.hit, wb.counts + bounce,
+                          cursors + bounce, wb.stats, QueryArgs{});
         }
         {
             Timed t(L, 1);
@@ -1432,21 +1432,9 @@ cudaError_t wf_first_rays(const Launcher& L, const FrameParams& fp, int mode, fl
 cudaError_t wf_query(const Launcher& L, const SceneView& sc, const QueryArgs& q, int64_t n, Query mode,
                      uint32_t* counts, unsigned long long* stats) {
     if (n <= 0) return cudaSuccess;
-    const bool wide = sc.nodes4 != nullptr, any = mode == Query::ANY;
-    const int grid = L.query_grid[any ? 1 : 0][wide ? 1 : 0];
-    k_hook_count<<<1, 32, 0, L.st>>>(counts, (uint32_t)n);
-    const PathArrays none{nullptr, nullptr, nullptr};
-#define RT_Q(C, W, QQ) k_extend<C, W, true, QQ><<<grid, kExtBlock, 0, L.st>>>(sc, none, nullptr, counts, counts + 1, stats, q)
-    if (any) {
-        if (wide) { if (L.instrument) RT_Q(true, true, Query::ANY); else RT_Q(false, true, Query::ANY); }
-        else { if (L.instrument) RT_Q(true, false, Query::ANY); else RT_Q(false, false, Query::ANY); }
-    } else {
-        if (wide) { if (L.instrument) RT_Q(true, true, Query::CLOSEST); else RT_Q(false, true, Query::CLOSEST); }
-        else { if (L.instrument) RT_Q(true, false, Query::CLOSEST); else RT_Q(false, false, Query::CLOSEST); }
-    }
-#undef RT_Q
-    (*L.kernel_launches) += 2;
-    (*L.extend_launches)++;
+    k_query_reset<<<1, 32, 0, L.st>>>(counts, (uint32_t)n);
+    (*L.kernel_launches)++;
+    launch_extend(L, sc, true, mode, PathArrays{nullptr, nullptr, nullptr}, nullptr, counts, counts + 1, stats, q);
     return cudaGetLastError();
 }
 
